@@ -15,7 +15,7 @@ value / e2e / roofline / clocks, at the same number of GPUs -- and a `parity` bl
 solved to convergence once on the same problem, compared with what the GPU arm returned.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--config c2|c2s|c3|c4|c4m|c4s|c5] [--extras default|all|none]
+                  [--config c2|c2s|c3|c4|c4m|c4s|c5] [--extras default|all|none] [--dump-outputs DIR]
 
   c2   mrcal-shaped calibration, Nstate 1268, Nmeas 1e6 (default)      c3  100 000 batched dense 256x16
   c4   bundle adjustment, 10 k cameras x 1 M points (c4m / c4s: 1/10, 1/100 scale)
@@ -324,7 +324,17 @@ def workload_name(cfg):
     return f"mrcal-shaped sparse calibration ({cfg}): {ncam} cams x {nframes} frames x {npts} points"
 
 
-def bench_c3(args, rank, world, local, dist):
+def dump_outputs(args, **arrays):
+    """--dump-outputs: what the last timed step returned to its caller, one DIR/<name>.npy per array (float64),
+    so that two builds can be compared output for output on identical, seeded inputs."""
+    if not args.dump_outputs:
+        return
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def bench_c3(args, rank, world, local, dist, brief=False):
     """Config C3: B independent dense problems (Nstate=16, Nmeas=256), split evenly over the GPUs
     (strong scaling, no data-path collective). One step = the whole batch solved once."""
     import torch
@@ -345,7 +355,7 @@ def bench_c3(args, rank, world, local, dist):
         rc, p, n2, it = H.solve_batched(dev, p0, N, M, max_iterations=100)
         assert rc == B
         L.dogleg_gpu_batched_stats(H.as_dp(st))
-        return int(it.sum()), st.copy(), float(n2.sum())
+        return it, st.copy(), p, n2
     for _ in range(args.warmup):
         solve()
     if dist is not None:
@@ -354,14 +364,15 @@ def bench_c3(args, rank, world, local, dist):
     sampler = ClockSampler(local)
     sampler.start()
     sampler.wait_first()
-    steps = min(args.steps, 20)
+    steps = min(args.steps, 20) if brief else args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     t0 = time.perf_counter()
     iters = launches = 0
     k_ms = cb_ms = trials = 0.0
     for _ in range(steps):
-        it, s, cost = solve()
+        it_each, s, p_last, n2_last = solve()
+        it = int(it_each.sum())
         iters += it
         launches += int(s[0])
         trials += s[1]
@@ -408,6 +419,8 @@ def bench_c3(args, rank, world, local, dist):
                              "algorithmic_bytes_per_launch": alg_per_trial * trials / max(launches, 1),
                              "avg_launch_ms": k_ms / max(launches, 1), "callback_ms_per_launch": cb_ms / max(launches, 1)},
                 "cpu_baseline": cpu}
+        if not brief:
+            dump_outputs(args, p=p_last, norm2x=n2_last, iterations=it_each)
     DL.dlb_dev_problem_free(dev)
     L.dogleg_gpu_release_cache()
     return line if rank == 0 else None
@@ -441,7 +454,7 @@ def measure_dgemm_peak():
     return _dgemm_peak[0]
 
 
-def bench_c5(args, rank, world, local, dist):
+def bench_c5(args, rank, world, local, dist, brief=False):
     """Config C5: one large dense problem (Nstate=4096, Nmeas=500k by default), Jacobian produced on
     the device; J'J on the DMMA SYRK kernel, blocked DMMA Cholesky. N > 1: the rows of J are split
     evenly over the ranks (dogleg_gpu_optimize_dense_sharded): every rank forms the J'J of its rows,
@@ -483,10 +496,11 @@ def bench_c5(args, rank, world, local, dist):
             r = L.dogleg_gpu_optimize_dense(H.as_dp(p), N, M, DL.dlb_dev_cb_dense_ptr(), C.c_void_p(dev), C.byref(P), None)
         assert r >= 0, L.dogleg_gpu_last_error()
         L.dogleg_gpu_get_stats(None, H.as_dp(st))
-        return r, st.copy()
-    for _ in range(min(args.warmup, 1)):
+        return r, st.copy(), p
+    warmup = min(args.warmup, 1) if brief else args.warmup
+    for _ in range(warmup):
         solve()
-    steps = min(args.steps, 3)
+    steps = min(args.steps, 3) if brief else args.steps
     if dist is not None:
         dist.barrier()
     sampler = ClockSampler(local)
@@ -498,7 +512,7 @@ def bench_c5(args, rank, world, local, dist):
     t0 = time.perf_counter()
     iters = launches = 0
     for _ in range(steps):
-        cost, s = solve()
+        cost, s, p_last = solve()
         iters += int(s[0])
         launches += int(s[4])
     e1.record()
@@ -511,7 +525,7 @@ def bench_c5(args, rank, world, local, dist):
     launches = int(barrier_sum(dist, launches))
     # per-phase device time of one more solve (events around every phase)
     os.environ["DOGLEG_GPU_PHASE_TIMING"] = "1"
-    _, s = solve()
+    _, s, _ = solve()
     os.environ["DOGLEG_GPU_PHASE_TIMING"] = "0"
     L.dogleg_gpu_get_phase_ms(H.as_dp(ph))
     if rank != 0:
@@ -525,7 +539,7 @@ def bench_c5(args, rank, world, local, dist):
     ach = flops / (syrk_ms * 1e-3) / 1e12
     names = ["h2d", "gradient", "cauchy_Jv", "assemble_syrk", "factor", "solve", "step_Jv", "d2h_p"]
     line = {"metric": "dogleg_iterations_per_sec", "value": iters / wall, "unit": "iterations/s", "n_gpus": world,
-            "steps": steps, "warmup": min(args.warmup, 1), "ms_per_step": 1e3 * wall / steps, "higher_is_better": True,
+            "steps": steps, "warmup": warmup, "ms_per_step": 1e3 * wall / steps, "higher_is_better": True,
             "scaling": "weak" if world == 1 else "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": {"workload": f"large dense (c5): Nstate={N}, Nmeas={M}", "iterations_per_solve": iters / steps,
                        "final_cost": cost, "callback": "device model kernel, included",
@@ -550,6 +564,8 @@ def bench_c5(args, rank, world, local, dist):
                                 "sample": f"REDUCED problem Nstate={Ns}, Nmeas={Ms} through the reference's dense path (rank-1 J'J + "
                                           f"dpptrf), capped at {args.ref_iterations} iterations; at full size one evaluation needs "
                                           "~40 min on one core (4.2e12 FMA at the measured 1.7 GFMA/s)"}
+    if not brief:
+        dump_outputs(args, p=p_last, norm2x=[cost])
     DL.dlb_dev_problem_free(dev)
     L.dogleg_gpu_release_cache()
     return line
@@ -929,6 +945,8 @@ def bench_sparse(args, cfg, rank, world, local, dist, brief=False, mode=None):
                 "clocks": clocks, "e2e": e2e, "gpu_launches": launches, "roofline": roof, "cpu_baseline": cpu}
         if parity is not None:
             line["parity"] = parity
+        if not brief:
+            dump_outputs(args, p=p_dev, norm2x=[cost])
         if sharded:
             cs = np.zeros(2)
             L.dogleg_gpu_get_comm_stats(H.as_dp(cs))
@@ -966,7 +984,12 @@ def main():
     ap.add_argument("--ref-iterations", type=int, default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-only", action="store_true", help="short run for ncu: no e2e, no cpu baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline config returned (final p, cost; c3: per "
+                         "problem, iterations too) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs at least one timed step")
     rank, world, local, dist = dist_setup(args.gpus)
     headline = args.config or "c2"
     if args.config is None:
@@ -981,9 +1004,9 @@ def main():
 
     def run(cfg, brief):
         if cfg == "c3":
-            return bench_c3(args, rank, world, local, dist)
+            return bench_c3(args, rank, world, local, dist, brief=brief)
         if cfg == "c5":
-            return bench_c5(args, rank, world, local, dist)
+            return bench_c5(args, rank, world, local, dist, brief=brief)
         if world > 1 and CONFIGS[cfg][0] != "ba":
             # a C2-sized iteration (0.4 ms, half of it a dependency chain that does not shard) gains nothing from being
             # split: the whole-job throughput of N GPUs is N solves at a time; the sharded solve rides along

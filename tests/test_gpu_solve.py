@@ -185,19 +185,21 @@ def test_rejected_steps_and_far_start(H, mode, p0):
     assert abs(got.norm2x - ref.norm2x) <= COST_RTOL * ref.norm2x
 
 
-def test_vnlog_output_matches_reference_text(H, tmp_path):
-    """The reference's own sample program, unchanged, linked against libdogleg.so: its vnlog
-    convergence log must equal the golden log field for field (SURVEY.md 4.1)."""
-    exe = os.path.join(ROOT, "oracle", "_ref", "sample_product")
-    if not os.path.exists(exe):
-        pytest.skip("sample_product was not built (needs /root/reference at build time)")
+def test_vnlog_output_matches_reference_text(H, capfd):
+    """The vnlog convergence log libdogleg.so prints for the reference's sample problem (sample.c's data and
+    start, max_iterations 8, DOGLEG_DEBUG_VNLOG) must equal the log the reference's own `sample --diag vnlog`
+    printed, field for field (SURVEY.md 4.1; tests/golden/sample_reference.json)."""
+    import ctypes as C
     gold = json.load(open(os.path.join(GOLD, "sample_reference.json")))
-    for mode, arg in [("sparse", "sparse"), ("dense", "dense"),
-                      ("products-packed-upper", "dense-products-packed-upper"),
-                      ("products-unpacked", "dense-products-unpacked")]:
-        out = subprocess.run([exe, "--diag", "vnlog", arg], capture_output=True, text=True)
-        assert out.returncode == 0, out.stderr
-        got = [l.split() for l in out.stdout.strip().splitlines()]
+    libc = C.CDLL(None)
+    for mode in ["sparse", "dense", "products-packed-upper", "products-unpacked"]:
+        libc.fflush(None)                              # the library prints with stdio
+        capfd.readouterr()
+        r = H.solve_product(H.Problem.sample(), mode, max_iterations=8, vnlog=True)
+        libc.fflush(None)
+        out = capfd.readouterr().out
+        assert r.norm2x >= 0
+        got = [l.split() for l in out.strip().splitlines()]
         want = [l.split() for l in gold[mode]["vnlog"].strip().splitlines()]
         assert got[0] == want[0]                       # legend
         assert len(got) == len(want)
@@ -207,8 +209,7 @@ def test_vnlog_output_matches_reference_text(H, tmp_path):
                 if a == b:
                     continue
                 assert np.isclose(float(a), float(b), rtol=2e-5), (g, w)   # %g prints 6 digits
-        chk = subprocess.run([exe, "--check", arg], capture_output=True, text=True)
-        assert chk.returncode == 0 and "ERROR" not in chk.stdout
+        assert np.max(np.abs(r.p - np.arange(1, 7))) < 5e-2          # what `sample --check` asserts
 
 
 def test_streaming_host_callback_gives_identical_results(H):
@@ -232,11 +233,15 @@ def test_streaming_host_callback_gives_identical_results(H):
 def test_full_size_mrcal_problem_matches_the_reference(H):
     """VERDICT round 1, weak #1: the FULL C2 problem (Nstate 1268, Nmeas 1e6, 22.5 M nonzeros) through
     dogleg_optimize2 with host callbacks against the unmodified reference on the same inputs: same number
-    of evaluations, cost to 1e-9, p to 1e-7 (the reference needs ~15 s on one host core)."""
-    if H.reference_lib() is None:
-        pytest.skip("oracle/_ref/libdogleg_ref.so is not built")
+    of evaluations, cost to 1e-9, p to 1e-7 (the reference needs ~15 s on one host core). Without the
+    reference, p comes from the oracle restatement, which must itself reproduce the reference's recorded
+    evaluation count and cost (tests/golden/c2_reference.json)."""
+    gold = json.load(open(os.path.join(GOLD, "c2_reference.json")))
     prob = H.Problem.mrcal(4, 200, 625, seed=2)
-    ref = H.solve_reference(prob, "sparse", max_iterations=100)
+    ref = H.solve_reference(prob, "sparse", max_iterations=100) if H.reference_lib() is not None \
+        else H.solve_oracle(prob, "sparse", max_iterations=100)
+    assert ref.ncalls == gold["ncalls"]
+    assert abs(ref.norm2x - gold["norm2x"]) <= COST_RTOL * gold["norm2x"]
     got = H.solve_product(prob, "sparse", max_iterations=100)
     assert got.ncalls == ref.ncalls
     assert abs(got.norm2x - ref.norm2x) <= COST_RTOL * abs(ref.norm2x)
