@@ -52,6 +52,17 @@ double dogleg_gpu_optimize_dense(double* p, unsigned int Nstate, unsigned int Nm
                                  const dogleg_parameters2_t* parameters,
                                  dogleg_solverContext_t** returnContext);
 
+/* dogleg_optimize_dense_products with the products produced on the device: d_norm2x is one double,
+ * d_Jtx Nstate doubles, d_JtJ the layout parameters->JtJ_packed / JtJ_upper select (Nstate*Nstate
+ * row-first, or Nstate*(Nstate+1)/2 packed upper, row-first). Packed lower is rejected before the first
+ * callback (the reference cannot take a Cauchy step with it, dogleg.c:597-601). */
+typedef void (dogleg_gpu_callback_dense_products_t)(const double* d_p, double* d_norm2x, double* d_Jtx,
+                                                     double* d_JtJ, void* stream, void* cookie);
+double dogleg_gpu_optimize_dense_products(double* p, unsigned int Nstate,
+                                          dogleg_gpu_callback_dense_products_t* f, void* cookie,
+                                          const dogleg_parameters2_t* parameters,
+                                          dogleg_solverContext_t** returnContext);
+
 /* ----------------------------------------- using the factorization of a returned context */
 /* The reference lets a returnContext caller solve with ctx->factorization through CHOLMOD
  * (dogleg.h:188-195, README.pod:105-111; dogleg.c:853-856 is how the library does it itself). Here the
@@ -147,10 +158,25 @@ int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate, unsigned i
                                       const dogleg_parameters2_t* parameters,
                                       double* norm2x_out, int* iterations_out);
 
-/* statistics of this thread's last batched solve: [0] trial launches, [1] sum over launches of
+/* B independent dense-products problems: the callback fills, for every active problem b,
+ * d_norm2x[b], d_Jtx[b*Nstate ..] and its JtJ at d_JtJ + b*S, S = Nstate*Nstate (row-first, both
+ * triangles) or Nstate*(Nstate+1)/2 (packed upper, row-first: parameters->JtJ_packed && JtJ_upper).
+ * Packed lower is rejected (the reference cannot take a Cauchy step with it, dogleg.c:597-601).
+ * No Jacobian is stored, so the batch size does not depend on the number of measurements.
+ * d_active[b]==0: finished, outputs ignored. Nstate <= 32. Return value, p, norm2x_out and
+ * iterations_out as dogleg_gpu_optimize_dense_batched. */
+typedef void (dogleg_gpu_callback_dense_products_batched_t)(const double* d_p, double* d_norm2x, double* d_Jtx,
+                                                             double* d_JtJ, const int* d_active, int B,
+                                                             void* stream, void* cookie);
+int dogleg_gpu_optimize_dense_products_batched(double* p, unsigned int Nstate, unsigned int B,
+                                               dogleg_gpu_callback_dense_products_batched_t* f, void* cookie,
+                                               const dogleg_parameters2_t* parameters,
+                                               double* norm2x_out, int* iterations_out);
+
+/* statistics of this thread's last batched solve (either form): [0] trial launches, [1] sum over launches of
  * active problems, [2] ms inside the trial kernel, [3] ms inside the callback (CUDA events) */
 void dogleg_gpu_batched_stats(double out[8]);
-/* the device workspace of the last batched solve is kept for the next one of the same shape;
+/* the device workspace of the last batched solve is kept for the next one of the same shape and form;
  * this frees it (dogleg_gpu_release_cache() does too) */
 void dogleg_gpu_release_batched_cache(void);
 
@@ -265,7 +291,8 @@ int           dlb_engine_pattern_equals(const dlb_engine_t* e, const int* Jp, co
 
 /* pinned host mirrors the engine owns (what dogleg_operatingPoint_t points at) */
 enum { DLB_BUF_P = 0, DLB_BUF_X = 1, DLB_BUF_JTX = 2, DLB_BUF_CAUCHY = 3, DLB_BUF_GN = 4,
-       DLB_BUF_STEP = 5, DLB_BUF_JVALUES = 6, DLB_BUF_JP = 7, DLB_BUF_JI = 8 };
+       DLB_BUF_STEP = 5, DLB_BUF_JVALUES = 6, DLB_BUF_JP = 7, DLB_BUF_JI = 8,
+       DLB_BUF_NORM2X = 9   /* device only, DENSE_PRODUCTS: the |x|^2 a device callback writes */ };
 void*         dlb_engine_host_buffer(dlb_engine_t* e, int slot, int which);
 /* raw device pointers of the same (for device callbacks and for wrapping as
  * tensors in the multi-GPU reduce); DLB_BUF_JVALUES .. only */
@@ -282,7 +309,8 @@ const dlb_symbolic_t* dlb_engine_symbolic(const dlb_engine_t* e);
 /* a15: H2D of x and Jacobian values from the slot's pinned mirrors (skipped if
  * from_host==0: a device callback already filled them), then Jt*x, |x|^2,
  * |Jt x|^2, max|Jt x| in one pass (dogleg.c:1025-1027, 1073-1081). For
- * DENSE_PRODUCTS norm2_x is taken from norm2x_products. */
+ * DENSE_PRODUCTS norm2_x is taken from norm2x_products (from_host) or from the
+ * slot's DLB_BUF_NORM2X device buffer (from_host==0). */
 int  dlb_engine_evaluate(dlb_engine_t* e, int slot, int from_host, double norm2x_products);
 /* called right before a host callback writes the slot's pinned buffers: arms dogleg_gpu_host_progress() */
 void dlb_engine_begin_host_fill(dlb_engine_t* e, int slot);

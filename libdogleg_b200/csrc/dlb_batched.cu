@@ -18,6 +18,12 @@
 // DENSE_PRODUCTS path does (dogleg.c:582-596, 1131-1155), so a rejected step needs only the
 // 2 KB JtJ of the current point (kept in HBM), never its 32 KB Jacobian. All reductions have a
 // fixed order; there are no block-wide barriers.
+//
+// Dense-products form (dogleg_gpu_optimize_dense_products_batched): the callback hands over |x|^2,
+// J'x and J'J itself (full, or the packed upper triangle), the reference's DOGLEG_DENSE_PRODUCTS
+// inputs (dogleg.c:1004-1083). The same kernel, instantiated with PRODUCTS, replaces the pass over J by a
+// coalesced load of those ~8(N^2 + N + 1) bytes per problem; everything from accept / reject on is
+// shared code. No J is ever stored, so the batch size no longer depends on Nmeas.
 #include "dlb_common.cuh"
 #include "dogleg_gpu.h"
 #include <vector>
@@ -44,6 +50,11 @@ struct BatchState
   double *x;            // B x M
   double *J;            // B x M x N
   int *n_active;
+  // dense-products callback buffers (appended: the dense instantiations keep their parameter offsets)
+  double *norm2x_in;    // B
+  double *Jtx_in;       // B x N
+  double *JtJ_in;       // B x N*N, or B x N(N+1)/2 packed upper row-first
+  int packed;
 };
 enum { FL_CAUCHY = 1, FL_GN = 2, FL_EDGE = 4, FL_PENDING = 8 };
 
@@ -82,8 +93,12 @@ __device__ __forceinline__ void bt_warp_sum2_all(double& a, double& b)
   for(int o = 16; o > 0; o >>= 1) { a += __shfl_xor_sync(0xffffffffu, a, o); b += __shfl_xor_sync(0xffffffffu, b, o); }
 }
 
-template<int NT8, int RING>
-__global__ void __launch_bounds__(BT_NT, NT8 <= 2 ? 3 : 1)
+// Blocks per SM the register budget is sized for: three for small dense problems (80 registers). The
+// products form at NT8 == 2 spills at 80 registers; it gets two blocks (119 registers, no spills).
+template<int NT8, bool PRODUCTS> constexpr int bt_min_blocks() { return NT8 == 1 ? 3 : NT8 == 2 ? (PRODUCTS ? 2 : 3) : 1; }
+
+template<int NT8, int RING, bool PRODUCTS>
+__global__ void __launch_bounds__(BT_NT, bt_min_blocks<NT8, PRODUCTS>())
 k_batched_trial(BatchState S)
 {
   extern __shared__ double sm[];
@@ -101,94 +116,122 @@ k_batched_trial(BatchState S)
   double* sn  = sc + BT_NMAX;              // gauss-newton
   double* ss  = sn + BT_NMAX;              // step
   double* sp  = ss + BT_NMAX;              // scratch
-  const int g = lane >> 2, tt = lane & 3;
-
-  // ---- one pass over the trial point's Jacobian: JtJ, J'x, |x|^2 ----
-  const double* gJ = S.J + (size_t)b * M * N;
-  const double* gx = S.x + (size_t)b * M;
-  double acc[NPAIR][2], ag[NT8][2];
-#pragma unroll
-  for(int i = 0; i < NPAIR; i++) { acc[i][0] = 0.0; acc[i][1] = 0.0; }
-#pragma unroll
-  for(int i = 0; i < NT8; i++) { ag[i][0] = 0.0; ag[i][1] = 0.0; }
-  double n2 = 0.0;
-  // one 4-row group: this lane's entries of the group's rows (zeros beyond the last row)
-  auto load_group = [&](int r0, double (&v)[NT8], double& xr) {
-    const int row = r0 + tt;
-    const bool valid = row < M;
-    xr = valid ? ldg_stream(gx + row) : 0.0;
-#pragma unroll
-    for(int ti = 0; ti < NT8; ti++) v[ti] = (valid && 8 * ti + g < N) ? ldg_stream(gJ + (size_t)row * N + 8 * ti + g) : 0.0;
-  };
-  auto use_group = [&](const double (&v)[NT8], double xr) {
-    // J'x by plain multiply-adds (this lane's row of the group times its x; the four lanes of a state are
-    // folded after the loop): as a DMMA it cost a third of the FP64 pipe, which this kernel loads almost
-    // as heavily as HBM (2.5 FMA per byte streamed against 2.9 FMA per byte of machine balance).
-    // Measured in round 2 (profiles/r02_variants.txt): 1.40 -> 1.35 ms per trial launch; splitting the kernel
-    // into a streaming pass and a step kernel (1.39-1.47 ms) and deeper register rings (6: 1.58 ms,
-    // 8: 1.61 ms) were slower and are not kept.
-    const double bx = g == 0 ? xr : 0.0;
-    int idx = 0;
-#pragma unroll
-    for(int ti = 0; ti < NT8; ti++)
-    {
-#pragma unroll
-      for(int tj = 0; tj <= ti; tj++, idx++) bt_dmma(acc[idx][0], acc[idx][1], v[ti], v[tj]);
-      ag[ti][0] = fma(v[ti], xr, ag[ti][0]);
-    }
-    n2 = fma(bx, bx, n2);
-  };
-  if(RING > 1)
-  { // register ring: the loads of group i + RING are issued before the DMMAs of group i, so RING
-    // groups (3 * RING loads per lane) are in flight; groups are consumed in the same order as
-    // below, hence bit-identical sums. Groups past the end are zeros.
-    double vb[RING > 1 ? RING : 1][NT8], xb[RING > 1 ? RING : 1];
-#pragma unroll
-    for(int u = 0; u < RING; u++) load_group(4 * u, vb[u], xb[u]);
-    for(int r0 = 0; r0 < M; r0 += 4 * RING)
-    {
-#pragma unroll
-      for(int u = 0; u < RING; u++)
+  double n2x_new;
+  if constexpr(PRODUCTS)
+  { // ---- the callback's products of the trial point: JtJ staged in sL (both triangles), J'x in sgn ----
+    if(S.packed)
+    { // packed upper, row-first: row r holds columns r..N-1 from offset r0. Consecutive lanes read
+      // consecutive entries; each lane walks its row index forward as its entry index grows.
+      const double* gP = S.JtJ_in + (size_t)b * (N * (N + 1) / 2);
+      int r = 0, r0 = 0;
+      for(int e = lane; e < N * (N + 1) / 2; e += 32)
       {
-        double v[NT8];
-#pragma unroll
-        for(int ti = 0; ti < NT8; ti++) v[ti] = vb[u][ti];
-        const double xr = xb[u];
-        load_group(r0 + 4 * (u + RING), vb[u], xb[u]);
-        use_group(v, xr);
+        while(e >= r0 + N - r) { r0 += N - r; r++; }
+        const int c = r + (e - r0);
+        const double val = ldg_stream(gP + e);
+        sL[r * LD + c] = val; sL[c * LD + r] = val;
       }
     }
+    else
+    {
+      const double* gF = S.JtJ_in + (size_t)b * N * N;
+      for(int e = lane; e < N * N; e += 32) { const int a = e / N, c = e - a * N; sL[a * LD + c] = ldg_stream(gF + e); }
+    }
+    if(lane < N) sgn[lane] = ldg_stream(S.Jtx_in + (size_t)b * N + lane);
+    n2x_new = S.norm2x_in[b];
+    (void)M;
   }
   else
   {
-#pragma unroll 8
-    for(int r0 = 0; r0 < M; r0 += 4)
-    {
-      double v[NT8], xr;
-      load_group(r0, v, xr);
-      use_group(v, xr);
-    }
-  }
+    const int g = lane >> 2, tt = lane & 3;
+
+    // ---- one pass over the trial point's Jacobian: JtJ, J'x, |x|^2 ----
+    const double* gJ = S.J + (size_t)b * M * N;
+    const double* gx = S.x + (size_t)b * M;
+    double acc[NPAIR][2], ag[NT8][2];
 #pragma unroll
-  for(int ti = 0; ti < NT8; ti++)
-  {
-    ag[ti][0] += __shfl_xor_sync(0xffffffffu, ag[ti][0], 1);
-    ag[ti][0] += __shfl_xor_sync(0xffffffffu, ag[ti][0], 2);
-  }
-  const double n2x_new = warp_sum_all(n2);
-  {
-    int idx = 0;
+    for(int i = 0; i < NPAIR; i++) { acc[i][0] = 0.0; acc[i][1] = 0.0; }
+#pragma unroll
+    for(int i = 0; i < NT8; i++) { ag[i][0] = 0.0; ag[i][1] = 0.0; }
+    double n2 = 0.0;
+    // one 4-row group: this lane's entries of the group's rows (zeros beyond the last row)
+    auto load_group = [&](int r0, double (&v)[NT8], double& xr) {
+      const int row = r0 + tt;
+      const bool valid = row < M;
+      xr = valid ? ldg_stream(gx + row) : 0.0;
+#pragma unroll
+      for(int ti = 0; ti < NT8; ti++) v[ti] = (valid && 8 * ti + g < N) ? ldg_stream(gJ + (size_t)row * N + 8 * ti + g) : 0.0;
+    };
+    auto use_group = [&](const double (&v)[NT8], double xr) {
+      // J'x by plain multiply-adds (this lane's row of the group times its x; the four lanes of a state are
+      // folded after the loop): as a DMMA it cost a third of the FP64 pipe, which this kernel loads almost
+      // as heavily as HBM (2.5 FMA per byte streamed against 2.9 FMA per byte of machine balance).
+      // Measured in round 2 (profiles/r02_variants.txt): 1.40 -> 1.35 ms per trial launch; splitting the kernel
+      // into a streaming pass and a step kernel (1.39-1.47 ms) and deeper register rings (6: 1.58 ms,
+      // 8: 1.61 ms) were slower and are not kept.
+      const double bx = g == 0 ? xr : 0.0;
+      int idx = 0;
+#pragma unroll
+      for(int ti = 0; ti < NT8; ti++)
+      {
+#pragma unroll
+        for(int tj = 0; tj <= ti; tj++, idx++) bt_dmma(acc[idx][0], acc[idx][1], v[ti], v[tj]);
+        ag[ti][0] = fma(v[ti], xr, ag[ti][0]);
+      }
+      n2 = fma(bx, bx, n2);
+    };
+    if(RING > 1)
+    { // register ring: the loads of group i + RING are issued before the DMMAs of group i, so RING
+      // groups (3 * RING loads per lane) are in flight; groups are consumed in the same order as
+      // below, hence bit-identical sums. Groups past the end are zeros.
+      double vb[RING > 1 ? RING : 1][NT8], xb[RING > 1 ? RING : 1];
+#pragma unroll
+      for(int u = 0; u < RING; u++) load_group(4 * u, vb[u], xb[u]);
+      for(int r0 = 0; r0 < M; r0 += 4 * RING)
+      {
+#pragma unroll
+        for(int u = 0; u < RING; u++)
+        {
+          double v[NT8];
+#pragma unroll
+          for(int ti = 0; ti < NT8; ti++) v[ti] = vb[u][ti];
+          const double xr = xb[u];
+          load_group(r0 + 4 * (u + RING), vb[u], xb[u]);
+          use_group(v, xr);
+        }
+      }
+    }
+    else
+    {
+#pragma unroll 8
+      for(int r0 = 0; r0 < M; r0 += 4)
+      {
+        double v[NT8], xr;
+        load_group(r0, v, xr);
+        use_group(v, xr);
+      }
+    }
 #pragma unroll
     for(int ti = 0; ti < NT8; ti++)
     {
+      ag[ti][0] += __shfl_xor_sync(0xffffffffu, ag[ti][0], 1);
+      ag[ti][0] += __shfl_xor_sync(0xffffffffu, ag[ti][0], 2);
+    }
+    n2x_new = warp_sum_all(n2);
+    {
+      int idx = 0;
 #pragma unroll
-      for(int tj = 0; tj <= ti; tj++, idx++)
+      for(int ti = 0; ti < NT8; ti++)
       {
-        const int a = 8 * ti + g, c0 = 8 * tj + 2 * tt;
-        sL[a * LD + c0] = acc[idx][0]; sL[a * LD + c0 + 1] = acc[idx][1];       // trial-point JtJ staged in sL
-        if(ti != tj) { sL[c0 * LD + a] = acc[idx][0]; sL[(c0 + 1) * LD + a] = acc[idx][1]; }
+#pragma unroll
+        for(int tj = 0; tj <= ti; tj++, idx++)
+        {
+          const int a = 8 * ti + g, c0 = 8 * tj + 2 * tt;
+          sL[a * LD + c0] = acc[idx][0]; sL[a * LD + c0 + 1] = acc[idx][1];       // trial-point JtJ staged in sL
+          if(ti != tj) { sL[c0 * LD + a] = acc[idx][0]; sL[(c0 + 1) * LD + a] = acc[idx][1]; }
+        }
+        if(tt == 0) sgn[8 * ti + g] = ag[ti][0];
       }
-      if(tt == 0) sgn[8 * ti + g] = ag[ti][0];
     }
   }
   __syncwarp();
@@ -396,24 +439,27 @@ static size_t batched_smem_bytes(int N)
   return sizeof(double) * (size_t)BT_WARPS * (2 * 8 * nt8 * ld + 6 * BT_NMAX);
 }
 typedef void (*batched_kernel_t)(BatchState);
-static batched_kernel_t batched_kernel(int N)
+// what the callback hands over; the two products layouts differ in the size of the JtJ buffer
+enum { BF_DENSE = 0, BF_PRODUCTS_FULL = 1, BF_PRODUCTS_PACKED = 2 };
+static batched_kernel_t batched_kernel(int N, int form)
 {
   // register-ring variant of the J'J loop (BT_RING row groups in flight; measured in round 2,
-  // profiles/r02_variants.txt: 1.37 -> 1.20 ms per trial launch at C3)
+  // profiles/r02_variants.txt: 1.37 -> 1.20 ms per trial launch at C3). The products form has no such loop.
+  const bool products = form != BF_DENSE;
   switch((N + 7) / 8)
   {
-  case 1: return k_batched_trial<1, BT_RING>;
-  case 2: return k_batched_trial<2, BT_RING>;
-  case 3: return k_batched_trial<3, BT_RING>;
-  default: return k_batched_trial<4, BT_RING>;
+  case 1: return products ? k_batched_trial<1, BT_RING, true> : k_batched_trial<1, BT_RING, false>;
+  case 2: return products ? k_batched_trial<2, BT_RING, true> : k_batched_trial<2, BT_RING, false>;
+  case 3: return products ? k_batched_trial<3, BT_RING, true> : k_batched_trial<3, BT_RING, false>;
+  default: return products ? k_batched_trial<4, BT_RING, true> : k_batched_trial<4, BT_RING, false>;
   }
 }
 
-// Device workspace of the last batched solve, kept for the next one of the same shape (the big
+// Device workspace of the last batched solve, kept for the next one of the same shape and form (the big
 // cudaMalloc/cudaFree pairs cost far more than a solve); dogleg_gpu_release_batched_cache() frees it.
 struct BatchWorkspace
 {
-  int B = 0, N = 0, M = 0, device = -1;
+  int B = 0, N = 0, M = 0, form = -1, device = -1;
   std::vector<void*> allocs;
   cudaStream_t st = 0;
   int* h_active = 0;
@@ -424,7 +470,7 @@ struct BatchWorkspace
     allocs.clear();
     if(st) cudaStreamDestroy(st);
     if(h_active) cudaFreeHost(h_active);
-    st = 0; h_active = 0; B = N = M = 0; device = -1;
+    st = 0; h_active = 0; B = N = M = 0; form = -1; device = -1;
   }
 };
 static thread_local BatchWorkspace g_ws;
@@ -433,21 +479,12 @@ extern "C" void dogleg_gpu_release_batched_cache(void) { g_ws.release(); }
 #define CUB(call) do { cudaError_t _e = (call); if(_e != cudaSuccess) { \
   dlb_set_error((std::string(#call) + ": " + cudaGetErrorString(_e)).c_str()); goto fail; } } while(0)
 
-extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate, unsigned int Nmeas,
-                                                 unsigned int B, dogleg_gpu_callback_dense_batched_t* f,
-                                                 void* cookie, const dogleg_parameters2_t* parameters,
-                                                 double* norm2x_out, int* iterations_out)
+// the solve behind both batched entry points, after their argument checks; M = 0 for the products form
+static int batched_solve(int form, double* p, int N, int M, unsigned int B, void* f, void* cookie,
+                         const dogleg_parameters2_t* parameters, double* norm2x_out, int* iterations_out)
 {
-  if(dogleg_gpu_device_count() <= 0) { dlb_set_error("no CUDA device available: libdogleg-b200 has no CPU fallback"); return -1; }
-  if(!f || !p || B == 0) { dlb_set_error("dense_batched: bad arguments"); return -1; }
-  const int N = (int)Nstate, M = (int)Nmeas;
   const size_t smem = batched_smem_bytes(N);
-  if(N > BT_NMAX || N < 1)
-  {
-    dlb_set_error("dense_batched: needs Nstate <= 32; use dogleg_optimize_dense2 per problem for bigger ones");
-    return -1;
-  }
-  batched_kernel_t kern = batched_kernel(N);
+  batched_kernel_t kern = batched_kernel(N, form);
   dogleg_parameters2_t P;
   if(parameters) P = *parameters; else dogleg_getDefaultParameters(&P);
   cudaSetDevice(dogleg_gpu_get_device());
@@ -460,29 +497,34 @@ extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate,
   S.Jtx_thr = P.Jt_x_threshold; S.upd_thr = P.update_threshold; S.tr_thr = P.trustregion_threshold;
   BatchWorkspace& W = g_ws;
   int result = -1;
-  if(W.B != (int)B || W.N != N || W.M != M || W.device != dogleg_gpu_get_device())
+  if(W.B != (int)B || W.N != N || W.M != M || W.form != form || W.device != dogleg_gpu_get_device())
   {
     W.release();
     W.device = dogleg_gpu_get_device();
     const size_t bN = (size_t)B * N * sizeof(double), bd = (size_t)B * sizeof(double), bi = (size_t)B * sizeof(int);
-    const size_t sizes[18] = { bd, bd, bd, bd, bd, bd, bi, bi, bi, bN, bN, bN, bN, bN,
-                               (size_t)B * N * N * sizeof(double), (size_t)B * M * sizeof(double),
-                               (size_t)B * M * N * sizeof(double), sizeof(int) };
+    std::vector<size_t> sizes = { bd, bd, bd, bd, bd, bd, bi, bi, bi, bN, bN, bN, bN, bN,
+                                  (size_t)B * N * N * sizeof(double), sizeof(int) };
+    if(form == BF_DENSE) sizes.insert(sizes.end(), { (size_t)B * M * sizeof(double), (size_t)B * M * N * sizeof(double) });
+    else
+    {
+      const size_t nS = form == BF_PRODUCTS_PACKED ? (size_t)N * (N + 1) / 2 : (size_t)N * N;
+      sizes.insert(sizes.end(), { bd, bN, (size_t)B * nS * sizeof(double) });
+    }
     for(size_t bytes : sizes)
     {
       void* q = 0;
       if(cudaMalloc(&q, bytes ? bytes : 8) != cudaSuccess) { cudaGetLastError(); break; }
       W.allocs.push_back(q);
     }
-    if(W.allocs.size() != 18 ||
+    if(W.allocs.size() != sizes.size() ||
        cudaStreamCreateWithFlags(&W.st, cudaStreamNonBlocking) != cudaSuccess ||
        cudaHostAlloc((void**)&W.h_active, sizeof(int), cudaHostAllocDefault) != cudaSuccess)
     {
       W.release();
-      dlb_set_error("dense_batched: out of device memory");
+      dlb_set_error(form == BF_DENSE ? "dense_batched: out of device memory" : "dense_products_batched: out of device memory");
       return -1;
     }
-    W.B = (int)B; W.N = N; W.M = M;
+    W.B = (int)B; W.N = N; W.M = M; W.form = form;
   }
   {
     void** a = W.allocs.data();
@@ -490,7 +532,9 @@ extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate,
     S.expected = (double*)a[4]; S.lambda = (double*)a[5];
     S.steps = (int*)a[6]; S.flags = (int*)a[7]; S.active = (int*)a[8];
     S.p_before = (double*)a[9]; S.ptrial = (double*)a[10]; S.Jtx = (double*)a[11]; S.cauchy = (double*)a[12];
-    S.gn = (double*)a[13]; S.JtJ = (double*)a[14]; S.x = (double*)a[15]; S.J = (double*)a[16]; S.n_active = (int*)a[17];
+    S.gn = (double*)a[13]; S.JtJ = (double*)a[14]; S.n_active = (int*)a[15];
+    if(form == BF_DENSE) { S.x = (double*)a[16]; S.J = (double*)a[17]; }
+    else { S.norm2x_in = (double*)a[16]; S.Jtx_in = (double*)a[17]; S.JtJ_in = (double*)a[18]; S.packed = form == BF_PRODUCTS_PACKED; }
   }
   cudaStream_t st = W.st;
   int* h_active = W.h_active;
@@ -521,7 +565,11 @@ extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate,
     {
       g_batched_stats[0] += 1; g_batched_stats[1] += *h_active;
       cudaEventRecord(ev[0], st);
-      f(S.ptrial, S.x, S.J, S.active, (int)B, (void*)st, cookie);
+      if(form == BF_DENSE)
+        ((dogleg_gpu_callback_dense_batched_t*)f)(S.ptrial, S.x, S.J, S.active, (int)B, (void*)st, cookie);
+      else
+        ((dogleg_gpu_callback_dense_products_batched_t*)f)(S.ptrial, S.norm2x_in, S.Jtx_in, S.JtJ_in, S.active, (int)B,
+                                                            (void*)st, cookie);
       cudaEventRecord(ev[1], st);
       kern<<<(B + BT_WARPS - 1) / BT_WARPS, BT_NT, smem, st>>>(S);
       cudaEventRecord(ev[2], st);
@@ -541,4 +589,43 @@ extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate,
   result = (int)B - *h_active;
 fail:
   return result;
+}
+
+extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate, unsigned int Nmeas,
+                                                 unsigned int B, dogleg_gpu_callback_dense_batched_t* f,
+                                                 void* cookie, const dogleg_parameters2_t* parameters,
+                                                 double* norm2x_out, int* iterations_out)
+{
+  if(dogleg_gpu_device_count() <= 0) { dlb_set_error("no CUDA device available: libdogleg-b200 has no CPU fallback"); return -1; }
+  if(!f || !p || B == 0) { dlb_set_error("dense_batched: bad arguments"); return -1; }
+  const int N = (int)Nstate;
+  if(N > BT_NMAX || N < 1)
+  {
+    dlb_set_error("dense_batched: needs Nstate <= 32; use dogleg_optimize_dense2 per problem for bigger ones");
+    return -1;
+  }
+  return batched_solve(BF_DENSE, p, N, (int)Nmeas, B, (void*)f, cookie, parameters, norm2x_out, iterations_out);
+}
+
+extern "C" int dogleg_gpu_optimize_dense_products_batched(double* p, unsigned int Nstate, unsigned int B,
+                                                          dogleg_gpu_callback_dense_products_batched_t* f, void* cookie,
+                                                          const dogleg_parameters2_t* parameters,
+                                                          double* norm2x_out, int* iterations_out)
+{
+  if(dogleg_gpu_device_count() <= 0) { dlb_set_error("no CUDA device available: libdogleg-b200 has no CPU fallback"); return -1; }
+  if(!f || !p || B == 0) { dlb_set_error("dense_products_batched: bad arguments (needs p, a callback and B > 0)"); return -1; }
+  const int N = (int)Nstate;
+  if(N > BT_NMAX || N < 1)
+  {
+    dlb_set_error("dense_products_batched: needs 1 <= Nstate <= 32; use dogleg_gpu_optimize_dense_products per problem for bigger ones");
+    return -1;
+  }
+  const bool packed = parameters && parameters->JtJ_packed;
+  if(packed && !parameters->JtJ_upper)
+  { // dogleg.c:597-601: the reference cannot form the Cauchy step from a packed lower triangle
+    dlb_set_error("dense_products_batched: a packed JtJ must be the upper triangle (JtJ_upper); packed lower is not supported");
+    return -1;
+  }
+  return batched_solve(packed ? BF_PRODUCTS_PACKED : BF_PRODUCTS_FULL, p, N, 0, B, (void*)f, cookie, parameters,
+                       norm2x_out, iterations_out);
 }

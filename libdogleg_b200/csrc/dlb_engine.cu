@@ -603,6 +603,9 @@ extern "C" void* dlb_engine_device_buffer(dlb_engine_t* e, int s, int which)
   // gather mode: this rank's slice inside the full-size arrays
   case DLB_BUF_X:       return L.d_x ? L.d_x + (e->gather ? e->col_begin : 0) : NULL;
   case DLB_BUF_JVALUES: return L.d_J ? L.d_J + (e->gather ? e->slice_off : 0) : NULL;
+  // the entry behind the gradient (d_Jtx holds N + 1); dense-products engines are never sharded, which is
+  // the only other use of it
+  case DLB_BUF_NORM2X:  return e->type == DOGLEG_DENSE_PRODUCTS ? L.d_Jtx + e->N : NULL;
   }
   return NULL;
 }
@@ -1279,6 +1282,8 @@ extern "C" int dlb_engine_evaluate(dlb_engine_t* e, int s, int from_host, double
     {
       dlb_launch_vec_stats_Jtx(L.d_Jtx, e->N, e->d_part, e->d_counter, e->d_sc, e->sm_count, e->st);
       e->n_launch += 1;
+      // a device callback left |x|^2 in DLB_BUF_NORM2X
+      if(!from_host) CU(cudaMemcpyAsync(&e->d_sc->norm2_x, L.d_Jtx + e->N, sizeof(double), cudaMemcpyDeviceToDevice, e->st));
     }
     CU(cudaGetLastError());
     if(e->sharded && g_nccl.world > 1)
@@ -1292,7 +1297,7 @@ extern "C" int dlb_engine_evaluate(dlb_engine_t* e, int s, int from_host, double
   }
   if(e->type == DOGLEG_SPARSE && e->fused_eval) { if(wait_published(e)) return -1; }
   else if(sync_scalars(e)) return -1;
-  if(e->type == DOGLEG_DENSE_PRODUCTS) e->h_sc->norm2_x = norm2x_products;
+  if(e->type == DOGLEG_DENSE_PRODUCTS && from_host) e->h_sc->norm2_x = norm2x_products;
   L.norm2_x = e->h_sc->norm2_x;
   L.norm2_Jtx = e->h_sc->norm2_Jtx;
   return 0;

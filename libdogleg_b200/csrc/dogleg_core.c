@@ -172,8 +172,11 @@ static bool evaluate_point(bool* converged, dogleg_operatingPoint_t* point, dogl
     double* d_p = dlb_engine_device_buffer(pv->eng, s, DLB_BUF_P);
     double* d_x = dlb_engine_device_buffer(pv->eng, s, DLB_BUF_X);
     double* d_J = dlb_engine_device_buffer(pv->eng, s, DLB_BUF_JVALUES);
-    if(ctx->solve_type == DOGLEG_SPARSE) pv->f_gpu_sparse(d_p, d_x, d_J, dlb_engine_stream(pv->eng), ctx->cookie);
-    else                                 pv->f_gpu_dense (d_p, d_x, d_J, dlb_engine_stream(pv->eng), ctx->cookie);
+    if(ctx->solve_type == DOGLEG_SPARSE)     pv->f_gpu_sparse(d_p, d_x, d_J, dlb_engine_stream(pv->eng), ctx->cookie);
+    else if(ctx->solve_type == DOGLEG_DENSE) pv->f_gpu_dense (d_p, d_x, d_J, dlb_engine_stream(pv->eng), ctx->cookie);
+    else /* d_J holds the slot's JtJ */      pv->f_gpu_products(d_p, dlb_engine_device_buffer(pv->eng, s, DLB_BUF_NORM2X),
+                                                                dlb_engine_device_buffer(pv->eng, s, DLB_BUF_JTX), d_J,
+                                                                dlb_engine_stream(pv->eng), ctx->cookie);
   }
   else if(ctx->solve_type == DOGLEG_SPARSE)   { dlb_engine_begin_host_fill(pv->eng, s); ctx->f(point->p, point->x, point->Jt, ctx->cookie); }
   else if(ctx->solve_type == DOGLEG_DENSE)    { dlb_engine_begin_host_fill(pv->eng, s); ctx->f_dense(point->p, point->x, point->J_dense, ctx->cookie); }
@@ -720,8 +723,9 @@ static double optimize_common(double* p, unsigned int Nstate, unsigned int Nmeas
   if(gpu_callback)
   {
     pv->device_callbacks = 1;
-    if(type == DOGLEG_SPARSE) pv->f_gpu_sparse = (dogleg_gpu_callback_sparse_t*)gpu_callback;
-    else                      pv->f_gpu_dense  = (dogleg_gpu_callback_dense_t*)gpu_callback;
+    if(type == DOGLEG_SPARSE)     pv->f_gpu_sparse   = (dogleg_gpu_callback_sparse_t*)gpu_callback;
+    else if(type == DOGLEG_DENSE) pv->f_gpu_dense    = (dogleg_gpu_callback_dense_t*)gpu_callback;
+    else                          pv->f_gpu_products = (dogleg_gpu_callback_dense_products_t*)gpu_callback;
   }
   { const char* env = getenv("DOGLEG_GPU_CHECK_PATTERN"); pv->check_pattern = env && atoi(env) != 0; }
   if(type == DOGLEG_SPARSE && pending_perm && pending_perm_n == (int)Nstate)
@@ -862,6 +866,22 @@ double dogleg_gpu_optimize_dense(double* p, unsigned int Nstate, unsigned int Nm
 {
   if(!f) { SAY("dogleg_gpu_optimize_dense: need a callback"); return -1.0; }
   return optimize_common(p, Nstate, Nmeas, 0, DOGLEG_DENSE, NULL, (void*)f, NULL, NULL, 0, 0,
+                         cookie, parameters, returnContext);
+}
+double dogleg_gpu_optimize_dense_products(double* p, unsigned int Nstate,
+                                          dogleg_gpu_callback_dense_products_t* f, void* cookie,
+                                          const dogleg_parameters2_t* parameters, dogleg_solverContext_t** returnContext)
+{
+  if(returnContext) *returnContext = NULL;
+  const dogleg_parameters2_t* P = parameters ? parameters : &global_settings;
+  const char* err = NULL;
+  if(dogleg_gpu_device_count() <= 0) err = "no CUDA device available: libdogleg-b200 has no CPU fallback";
+  else if(!f || !p || Nstate == 0)   err = "dogleg_gpu_optimize_dense_products: need p, Nstate > 0 and a callback";
+  /* the reference accepts a packed lower JtJ and fails at the first Cauchy step (dogleg.c:597-601); refuse it
+   * before any evaluation instead */
+  else if(P->JtJ_packed && !P->JtJ_upper) err = "dogleg_gpu_optimize_dense_products: a packed JtJ must be the upper triangle (JtJ_upper)";
+  if(err) { dlb_set_error(err); SAY("ERROR: %s", err); return -1.0; }
+  return optimize_common(p, Nstate, 0, 0, DOGLEG_DENSE_PRODUCTS, NULL, (void*)f, NULL, NULL, 0, 0,
                          cookie, parameters, returnContext);
 }
 double dogleg_gpu_optimize_dense_sharded(double* p, unsigned int Nstate, unsigned int Nmeas_total,

@@ -16,6 +16,7 @@ typedef struct dlb_private
   int context_returned;
   dogleg_gpu_callback_sparse_t* f_gpu_sparse;
   dogleg_gpu_callback_dense_t*  f_gpu_dense;
+  dogleg_gpu_callback_dense_products_t* f_gpu_products;
   int pattern_set, pattern_slot, check_pattern;
   int have_user_perm, user_perm_postorder;
   int* user_perm;

@@ -8,7 +8,7 @@ ROOT = os.path.dirname(HERE)
 
 SOLVE_DENSE, SOLVE_SPARSE, SOLVE_DENSE_PRODUCTS = 0, 1, 2      # dogleg_solve_type_t
 DEBUG_VNLOG = 1 << 30
-BUF_P, BUF_X, BUF_JTX, BUF_CAUCHY, BUF_GN, BUF_STEP, BUF_JVALUES, BUF_JP, BUF_JI = range(9)
+BUF_P, BUF_X, BUF_JTX, BUF_CAUCHY, BUF_GN, BUF_STEP, BUF_JVALUES, BUF_JP, BUF_JI, BUF_NORM2X = range(10)
 STEP_CAUCHY, STEP_GAUSSNEWTON, STEP_INTERPOLATED = 0, 1, 2
 SYM = dict(perm=0, parent=1, colcount=2, sn_first=3, rows_ptr=4, rows=5, sn_parent=6,
            cls_of_col=7, cls_front=8, sn_level=9, rel=10, child_ptr=11, child_list=12, level_ptr=13,
@@ -112,6 +112,11 @@ def load():
     L.dogleg_gpu_optimize_dense.restype = C.c_double
     L.dogleg_gpu_optimize_dense_batched.argtypes = [dp, C.c_uint, C.c_uint, C.c_uint, vp, vp, PP, dp, ip]
     L.dogleg_gpu_optimize_dense_batched.restype = C.c_int
+    L.dogleg_gpu_optimize_dense_products.argtypes = [dp, C.c_uint, vp, vp, PP, C.POINTER(vp)]
+    L.dogleg_gpu_optimize_dense_products.restype = C.c_double
+    L.dogleg_gpu_optimize_dense_products_batched.argtypes = [dp, C.c_uint, C.c_uint, vp, vp, PP, dp, ip]
+    L.dogleg_gpu_optimize_dense_products_batched.restype = C.c_int
+    L.dogleg_gpu_release_batched_cache.restype = None
     L.dogleg_gpu_batched_stats.argtypes = [dp]
     L.dogleg_gpu_batched_stats.restype = None
     # row-sharded multi-GPU solves (NCCL inside the library)
