@@ -173,6 +173,58 @@ int dogleg_gpu_optimize_dense_products_batched(double* p, unsigned int Nstate, u
                                                const dogleg_parameters2_t* parameters,
                                                double* norm2x_out, int* iterations_out);
 
+/* ------------------------------------------- the final state of a batched solve */
+/* What a batched caller needs for per-problem uncertainties, the batched counterpart of returnContext +
+ * dogleg_gpu_solve: each problem's JtJ at the p it returned, its lambda and why it stopped. */
+typedef struct dogleg_gpu_batch dogleg_gpu_batch_t;
+
+/* dogleg_gpu_optimize_dense_batched / dogleg_gpu_optimize_dense_products_batched (those two are these with
+ * returnBatch == NULL). If returnBatch != NULL, *returnBatch receives a handle that holds each problem's final
+ * JtJ (at the returned p), its lambda and its termination status, on the device the solve ran on;
+ * *returnBatch = NULL on failure. Free it with dogleg_gpu_batch_free(). The handle owns its memory: later
+ * batched solves, dogleg_gpu_release_batched_cache() and dogleg_gpu_release_cache() do not touch it. */
+int dogleg_gpu_optimize_dense_batched2(double* p, unsigned int Nstate, unsigned int Nmeas, unsigned int B,
+                                       dogleg_gpu_callback_dense_batched_t* f, void* cookie,
+                                       const dogleg_parameters2_t* parameters,
+                                       double* norm2x_out, int* iterations_out, dogleg_gpu_batch_t** returnBatch);
+int dogleg_gpu_optimize_dense_products_batched2(double* p, unsigned int Nstate, unsigned int B,
+                                                dogleg_gpu_callback_dense_products_batched_t* f, void* cookie,
+                                                const dogleg_parameters2_t* parameters,
+                                                double* norm2x_out, int* iterations_out,
+                                                dogleg_gpu_batch_t** returnBatch);
+
+/* Why a problem stopped, in the order the single-problem solver tests (dogleg_core.c run_solver): after an
+ * accepted step the gradient test comes before the iteration cap; at the initial point a problem is
+ * GRADIENT if it has converged, else MAX_ITERATIONS if max_iterations <= 0. */
+enum { DOGLEG_GPU_BATCH_UNFINISHED = 0,      /* still running when the solve stopped (trial cap) */
+       DOGLEG_GPU_BATCH_GRADIENT = 1,        /* max|J'x| <= Jt_x_threshold */
+       DOGLEG_GPU_BATCH_STEP = 2,            /* max|step| <= update_threshold: the step was not taken */
+       DOGLEG_GPU_BATCH_TRUSTREGION = 3,     /* rejected and trust region < trustregion_threshold */
+       DOGLEG_GPU_BATCH_MAX_ITERATIONS = 4 };
+
+/* Every call below works on JtJ_b + lambda_b I with the problem's sticky lambda at the end of its solve: the
+ * matrix dogleg_gpu_solve() uses on a returned context. A problem may have stopped without a Gauss-Newton
+ * step at its final point, so its JtJ can be singular; the factorization then climbs the solver's ladder
+ * (0 -> 1e-10 -> x10) and stores the raised lambda in the handle, as dogleg_computeJtJfactorization() does
+ * for ctx->lambda. Return 0 on success, < 0 with dogleg_gpu_last_error() set on bad arguments or a CUDA
+ * failure. A problem whose matrix is not positive definite at any lambda (non-finite entries) gets NaN
+ * outputs; the host-pointer forms return the number of such problems, the _device forms return 0 once the
+ * work is enqueued (they do not synchronise). */
+
+/* host arrays of B entries, either may be NULL; waits for the handle's pending work */
+int  dogleg_gpu_batch_status(const dogleg_gpu_batch_t* batch, int* status_out, double* lambda_out);
+/* X_b = (JtJ_b + lambda_b I)^-1 R_b for every problem. R, X: B x Nstate x nrhs, each problem's block
+ * column-major as in dogleg_gpu_solve. Host pointers; the _device form takes device pointers and enqueues on
+ * `stream` (a cudaStream_t, NULL = the legacy default stream) without synchronising. */
+int  dogleg_gpu_batch_solve(dogleg_gpu_batch_t* batch, const double* R, double* X, int nrhs);
+int  dogleg_gpu_batch_solve_device(dogleg_gpu_batch_t* batch, const double* d_R, double* d_X, int nrhs, void* stream);
+/* (JtJ_b + lambda_b I)^-1 for every problem: B x Nstate^2 (column k of problem b's block is the solve with
+ * e_k, so the layout reads as row-first and as column-first), or, if packed != 0, B x Nstate(Nstate+1)/2:
+ * the upper triangle of that row-first matrix, packed row-first (the products layout) */
+int  dogleg_gpu_batch_covariance(dogleg_gpu_batch_t* batch, double* out, int packed);
+int  dogleg_gpu_batch_covariance_device(dogleg_gpu_batch_t* batch, double* d_out, int packed, void* stream);
+void dogleg_gpu_batch_free(dogleg_gpu_batch_t** batch);   /* sets *batch = NULL; NULL is fine */
+
 /* statistics of this thread's last batched solve (either form): [0] trial launches, [1] sum over launches of
  * active problems, [2] ms inside the trial kernel, [3] ms inside the callback (CUDA events) */
 void dogleg_gpu_batched_stats(double out[8]);

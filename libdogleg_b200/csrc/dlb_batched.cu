@@ -24,6 +24,10 @@
 // inputs (dogleg.c:1004-1083). The same kernel, instantiated with PRODUCTS, replaces the pass over J by a
 // coalesced load of those ~8(N^2 + N + 1) bytes per problem; everything from accept / reject on is
 // shared code. No J is ever stored, so the batch size no longer depends on Nmeas.
+//
+// Final state (the `2` entry points with a dogleg_gpu_batch_t): the trial kernel also keeps the final point's
+// JtJ and writes why each problem stopped; k_batched_factor factors every problem's JtJ + lambda I with the
+// same ladder and solves with it (dogleg_gpu_batch_solve, dogleg_gpu_batch_covariance).
 #include "dlb_common.cuh"
 #include "dogleg_gpu.h"
 #include <vector>
@@ -55,6 +59,9 @@ struct BatchState
   double *Jtx_in;       // B x N
   double *JtJ_in;       // B x N*N, or B x N(N+1)/2 packed upper row-first
   int packed;
+  // a dogleg_gpu_batch_t was asked for (appended likewise): B termination codes (DOGLEG_GPU_BATCH_*), and the
+  // final point's JtJ is kept in JtJ. NULL: neither.
+  int *status;
 };
 enum { FL_CAUCHY = 1, FL_GN = 2, FL_EDGE = 4, FL_PENDING = 8 };
 
@@ -91,6 +98,50 @@ __device__ __forceinline__ void bt_warp_sum2_all(double& a, double& b)
 {
 #pragma unroll
   for(int o = 16; o > 0; o >>= 1) { a += __shfl_xor_sync(0xffffffffu, a, o); b += __shfl_xor_sync(0xffffffffu, b, o); }
+}
+
+// Cholesky of A + lambda I with the lambda ladder (dogleg.c:699-816), lane == row; A and the factor are
+// N x N, row stride 8 * NT8 + 1, in the warp's shared memory. The lane keeps ITS ROW of L in Lr; per pivot:
+// the diagonal comes by one shuffle, every lane forms rsqrt(d) itself (no sqrt -> division chain, DESIGN.md
+// divergence 7), the scaled column goes through shared memory once and the row updates are independent
+// multiply-adds. On return sL holds L (lower triangle, zeros above), Lr this lane's row of it, rsv the
+// reciprocal pivots (the same in every lane) and lam the lambda it took; lam is not finite if no lambda
+// of the ladder gave a positive definite matrix.
+template<int NT8>
+__device__ __forceinline__ void bt_cholesky_ladder(const double* sA, double* sL, int N, int lane, double& lam,
+                                                   double (&Lr)[8 * NT8], double (&rsv)[8 * NT8])
+{
+  constexpr int NMAX = 8 * NT8, LD = NMAX + 1;
+  for(;;)
+  {
+#pragma unroll
+    for(int c = 0; c < NMAX; c++)
+    {
+      const bool in = lane < N && c <= lane;
+      const double val = sA[(in ? lane : 0) * LD + (in ? c : 0)];
+      Lr[c] = in ? val + (c == lane ? lam : 0.0) : 0.0;
+    }
+    bool ok = true;
+#pragma unroll
+    for(int j = 0; j < NMAX; j++)
+    {
+      if(j >= N || !ok) continue;                    // (uniform)
+      const double d = __shfl_sync(0xffffffffu, Lr[j], j);
+      if(!(d > 0.0) || isinf(d)) { ok = false; continue; }
+      const double rs = rsqrt(d);
+      rsv[j] = rs;
+      Lr[j] = lane == j ? d * rs : Lr[j] * rs;       // (zero for the lanes above the pivot)
+      if(lane < N) sL[lane * LD + j] = Lr[j];
+      __syncwarp();
+#pragma unroll
+      for(int c = j + 1; c < NMAX; c++)
+        if(c <= lane && c < N) Lr[c] = fma(-Lr[j], sL[c * LD + j], Lr[c]);
+    }
+    if(ok) break;
+    lam = lam == 0.0 ? 1e-10 : lam * 10.0;             // dogleg.c:811-813
+    if(!isfinite(lam)) break;
+    __syncwarp();
+  }
 }
 
 // Blocks per SM the register budget is sized for: three for small dense problems (80 registers). The
@@ -271,7 +322,7 @@ k_batched_trial(BatchState S)
   if(accepted)
   { // the trial point becomes the current one: its JtJ and gradient are kept for retries
     flags &= ~(FL_CAUCHY | FL_GN | FL_EDGE);
-    for(int e = lane; e < N * N; e += 32) { const int a = e / N, c = e - a * N; const double val = sL[a * LD + c]; sA[a * LD + c] = val; if(!done) gA[e] = val; }
+    for(int e = lane; e < N * N; e += 32) { const int a = e / N, c = e - a * N; const double val = sL[a * LD + c]; sA[a * LD + c] = val; if(!done || S.status) gA[e] = val; }
     if(lane < N)
     {
       S.p_before[(size_t)b * N + lane] = S.ptrial[(size_t)b * N + lane];
@@ -293,7 +344,13 @@ k_batched_trial(BatchState S)
   if(lane == 0) { S.tr[b] = tr; S.steps[b] = steps; }
   if(done)
   {
-    if(lane == 0) { S.flags[b] = flags; S.active[b] = 0; atomicSub(S.n_active, 1); }
+    if(lane == 0)
+    {
+      S.flags[b] = flags; S.active[b] = 0; atomicSub(S.n_active, 1);
+      // the gradient test comes before the iteration cap (dogleg_core.c run_solver)
+      if(S.status) S.status[b] = !accepted ? DOGLEG_GPU_BATCH_TRUSTREGION
+                                           : converged ? DOGLEG_GPU_BATCH_GRADIENT : DOGLEG_GPU_BATCH_MAX_ITERATIONS;
+    }
     return;
   }
   __syncwarp();
@@ -321,44 +378,12 @@ k_batched_trial(BatchState S)
   {
     if(!(flags & FL_GN))
     {
-      // Cholesky of JtJ + lambda I with the lambda ladder (dogleg.c:699-816), lane == row. The lane keeps ITS ROW
-      // of L in registers; per pivot: the diagonal comes by one shuffle, every lane forms rsqrt(d) itself (no
-      // sqrt -> division chain, DESIGN.md divergence 7), the scaled column goes through shared memory once and
-      // the row updates are independent multiply-adds. The two substitutions multiply by the stored
-      // reciprocals and hand each solved entry round by one shuffle.
+      // Cholesky of JtJ + lambda I with the lambda ladder, lane == row. The two substitutions multiply by the
+      // stored reciprocals and hand each solved entry round by one shuffle.
       constexpr int NMAX = 8 * NT8;
       double lam = S.lambda[b];
       double Lr[NMAX], rsv[NMAX];
-      for(;;)
-      {
-#pragma unroll
-        for(int c = 0; c < NMAX; c++)
-        {
-          const bool in = lane < N && c <= lane;
-          const double val = sA[(in ? lane : 0) * LD + (in ? c : 0)];
-          Lr[c] = in ? val + (c == lane ? lam : 0.0) : 0.0;
-        }
-        bool ok = true;
-#pragma unroll
-        for(int j = 0; j < NMAX; j++)
-        {
-          if(j >= N || !ok) continue;                    // (uniform)
-          const double d = __shfl_sync(0xffffffffu, Lr[j], j);
-          if(!(d > 0.0) || isinf(d)) { ok = false; continue; }
-          const double rs = rsqrt(d);
-          rsv[j] = rs;
-          Lr[j] = lane == j ? d * rs : Lr[j] * rs;       // (zero for the lanes above the pivot)
-          if(lane < N) sL[lane * LD + j] = Lr[j];
-          __syncwarp();
-#pragma unroll
-          for(int c = j + 1; c < NMAX; c++)
-            if(c <= lane && c < N) Lr[c] = fma(-Lr[j], sL[c * LD + j], Lr[c]);
-        }
-        if(ok) break;
-        lam = lam == 0.0 ? 1e-10 : lam * 10.0;             // dogleg.c:811-813
-        if(!isfinite(lam)) break;
-        __syncwarp();
-      }
+      bt_cholesky_ladder<NT8>(sA, sL, N, lane, lam, Lr, rsv);
       if(lane == 0) S.lambda[b] = lam;
       // (JtJ + lambda I) u = Jt_x, gn = -u (dogleg.c:867-898)
       double yv = lane < N ? sg[lane] : 0.0;
@@ -422,9 +447,111 @@ k_batched_trial(BatchState S)
   {
     S.expected[b] = expected;
     S.flags[b] = flags | FL_PENDING;
-    if(finished) { S.active[b] = 0; atomicSub(S.n_active, 1); }
+    if(finished)
+    {
+      S.active[b] = 0; atomicSub(S.n_active, 1);
+      if(S.status) S.status[b] = DOGLEG_GPU_BATCH_STEP;
+    }
   }
   (void)sp;
+}
+
+// ---- solves with the final state of a batched solve (dogleg_gpu_batch_t) ----
+struct BatchFactorArgs
+{
+  int B, N, nrhs;             // nrhs: columns of R and X
+  const double* JtJ;          // B x N*N
+  double* lambda;             // B; raised in place by the ladder
+  const double* R;            // B x N x nrhs, column-major per problem; NULL: the identity (nrhs = N)
+  double* X;                  // like R; packed: B x N(N+1)/2, the upper triangle of the row-first result
+  int packed;
+  int* nfail;                 // counts the problems no lambda makes positive definite (may be NULL)
+};
+
+// One warp per problem: JtJ + lambda I factored by the trial kernel's ladder, then both substitutions with
+// lane == right-hand-side column, up to 32 columns at a time. L and the reciprocal pivots sit in the warp's
+// shared memory and every lane reads the same entry, so the reads are broadcasts and the chain is about N^2
+// multiply-adds for all 32 columns. Right-hand sides and results are staged through shared memory (column k
+// at sY[k * LD]) so that each problem's global reads and writes are coalesced. The sums run in the order of
+// the trial kernel's substitutions, so the solve with J'x reproduces its Gauss-Newton step bit for bit.
+template<int NT8>
+__global__ void __launch_bounds__(BT_NT) k_batched_factor(BatchFactorArgs A)
+{
+  extern __shared__ double sm[];
+  constexpr int NMAX = 8 * NT8, LD = NMAX + 1;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int b = blockIdx.x * BT_WARPS + w;
+  if(b >= A.B) return;
+  const int N = A.N;
+  double* sY  = sm + (size_t)w * (32 * LD + NMAX * LD + NMAX);   // JtJ, then right-hand sides / results
+  double* sL  = sY + 32 * LD;                                     // Cholesky factor
+  double* srs = sL + NMAX * LD;                                   // reciprocal pivots
+  const double* gA = A.JtJ + (size_t)b * N * N;
+  for(int e = lane; e < N * N; e += 32) { const int a = e / N, c = e - a * N; sY[a * LD + c] = ldg_stream(gA + e); }
+  double lam = A.lambda[b];
+  __syncwarp();
+  {
+    double Lr[NMAX], rsv[NMAX];
+    bt_cholesky_ladder<NT8>(sY, sL, N, lane, lam, Lr, rsv);
+#pragma unroll
+    for(int j = 0; j < NMAX; j++)
+      if(j < N && lane == j) srs[j] = rsv[j];
+  }
+  const bool failed = !isfinite(lam);
+  if(lane == 0) { A.lambda[b] = lam; if(failed && A.nfail) atomicAdd(A.nfail, 1); }
+  __syncwarp();
+
+  const int ncols = A.R ? A.nrhs : N;
+  const double* gR = A.R ? A.R + (size_t)b * N * ncols : nullptr;
+  double* gX = A.X + (A.packed ? (size_t)b * (N * (N + 1) / 2) : (size_t)b * N * ncols);
+  for(int c0 = 0; c0 < ncols; c0 += 32)
+  {
+    const int nc = min(32, ncols - c0);
+    if(gR)
+    {
+      for(int e = lane; e < nc * N; e += 32) { const int k = e / N, i = e - k * N; sY[k * LD + i] = ldg_stream(gR + (size_t)c0 * N + e); }
+      __syncwarp();
+    }
+    double y[NMAX];                                               // entries >= N are never read
+#pragma unroll
+    for(int i = 0; i < NMAX; i++) y[i] = gR ? sY[lane * LD + i] : (i == c0 + lane ? 1.0 : 0.0);
+#pragma unroll
+    for(int j = 0; j < NMAX; j++)                                 // L y = r
+    {
+      if(j >= N) continue;
+      double acc = y[j];
+#pragma unroll
+      for(int i = 0; i < j; i++) acc = fma(-sL[j * LD + i], y[i], acc);
+      y[j] = acc * srs[j];
+    }
+#pragma unroll
+    for(int j = NMAX - 1; j >= 0; j--)                            // L' x = y
+    {
+      if(j >= N) continue;
+      double acc = y[j];
+#pragma unroll
+      for(int i = NMAX - 1; i > j; i--)
+        if(i < N) acc = fma(-sL[i * LD + j], y[i], acc);
+      y[j] = acc * srs[j];
+    }
+    __syncwarp();
+#pragma unroll
+    for(int i = 0; i < NMAX; i++)
+      if(i < N) sY[lane * LD + i] = failed ? __longlong_as_double(0x7ff8000000000000LL) : y[i];
+    __syncwarp();
+    if(A.packed)
+    { // (covariance: one chunk) row r of the packed upper triangle = entries r..N-1 of column r
+      int r = 0, r0 = 0;
+      for(int e = lane; e < N * (N + 1) / 2; e += 32)
+      {
+        while(e >= r0 + N - r) { r0 += N - r; r++; }
+        gX[e] = sY[r * LD + r + (e - r0)];
+      }
+    }
+    else
+      for(int e = lane; e < nc * N; e += 32) { const int k = e / N, i = e - k * N; gX[(size_t)c0 * N + e] = sY[k * LD + i]; }
+    __syncwarp();
+  }
 }
 
 // statistics of the last batched solve of this thread, for bench.py:
@@ -479,9 +606,59 @@ extern "C" void dogleg_gpu_release_batched_cache(void) { g_ws.release(); }
 #define CUB(call) do { cudaError_t _e = (call); if(_e != cudaSuccess) { \
   dlb_set_error((std::string(#call) + ": " + cudaGetErrorString(_e)).c_str()); goto fail; } } while(0)
 
+// The final state of a batched solve. Its own allocations: the workspace cache never aliases them.
+struct dogleg_gpu_batch
+{
+  int device = -1, B = 0, N = 0;
+  double* JtJ = 0;            // B x N*N, the final point's
+  double* lambda = 0;         // B
+  int* status = 0;            // B, DOGLEG_GPU_BATCH_*
+  int* nfail = 0;             // 1, for the host-pointer forms
+  cudaStream_t st = 0;        // the host-pointer forms run here
+  cudaEvent_t ev = 0;         // the handle's last enqueued work: every call is ordered after it
+};
+
+// makes the handle's device current for the scope of a call and restores the caller's afterwards
+struct DeviceScope
+{
+  int prev = -1;
+  explicit DeviceScope(int d) { if(cudaGetDevice(&prev) != cudaSuccess) prev = -1; cudaSetDevice(d); }
+  ~DeviceScope() { if(prev >= 0) cudaSetDevice(prev); }
+};
+
+static void batch_destroy(dogleg_gpu_batch_t* h)
+{
+  DeviceScope ds(h->device);
+  if(h->ev) cudaEventSynchronize(h->ev);
+  cudaFree(h->JtJ); cudaFree(h->lambda); cudaFree(h->status); cudaFree(h->nfail);
+  if(h->st) cudaStreamDestroy(h->st);
+  if(h->ev) cudaEventDestroy(h->ev);
+  delete h;
+}
+
+static dogleg_gpu_batch_t* batch_create(int device, int B, int N)
+{
+  dogleg_gpu_batch_t* h = new dogleg_gpu_batch_t;
+  h->device = device; h->B = B; h->N = N;
+  DeviceScope ds(device);
+  if(cudaMalloc((void**)&h->JtJ, (size_t)B * N * N * sizeof(double)) != cudaSuccess ||
+     cudaMalloc((void**)&h->lambda, (size_t)B * sizeof(double)) != cudaSuccess ||
+     cudaMalloc((void**)&h->status, (size_t)B * sizeof(int)) != cudaSuccess ||
+     cudaMalloc((void**)&h->nfail, sizeof(int)) != cudaSuccess ||
+     cudaStreamCreateWithFlags(&h->st, cudaStreamNonBlocking) != cudaSuccess ||
+     cudaEventCreateWithFlags(&h->ev, cudaEventDisableTiming) != cudaSuccess)
+  {
+    cudaGetLastError();
+    batch_destroy(h);
+    return 0;
+  }
+  return h;
+}
+
 // the solve behind both batched entry points, after their argument checks; M = 0 for the products form
 static int batched_solve(int form, double* p, int N, int M, unsigned int B, void* f, void* cookie,
-                         const dogleg_parameters2_t* parameters, double* norm2x_out, int* iterations_out)
+                         const dogleg_parameters2_t* parameters, double* norm2x_out, int* iterations_out,
+                         dogleg_gpu_batch_t** returnBatch)
 {
   const size_t smem = batched_smem_bytes(N);
   batched_kernel_t kern = batched_kernel(N, form);
@@ -497,6 +674,7 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   S.Jtx_thr = P.Jt_x_threshold; S.upd_thr = P.update_threshold; S.tr_thr = P.trustregion_threshold;
   BatchWorkspace& W = g_ws;
   int result = -1;
+  dogleg_gpu_batch_t* h = 0;
   if(W.B != (int)B || W.N != N || W.M != M || W.form != form || W.device != dogleg_gpu_get_device())
   {
     W.release();
@@ -538,6 +716,18 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   }
   cudaStream_t st = W.st;
   int* h_active = W.h_active;
+  if(returnBatch)
+  {
+    h = batch_create(W.device, (int)B, N);
+    if(!h)
+    {
+      dlb_set_error(form == BF_DENSE ? "dense_batched2: out of device memory for the returned batch"
+                                     : "dense_products_batched2: out of device memory for the returned batch");
+      return -1;
+    }
+    S.status = h->status;
+    CUB(cudaMemsetAsync(S.status, 0, (size_t)B * sizeof(int), st));
+  }
   CUB(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   CUB(cudaMemcpyAsync(S.ptrial, p, (size_t)B * N * sizeof(double), cudaMemcpyHostToDevice, st));
   CUB(cudaMemcpyAsync(S.p_before, p, (size_t)B * N * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -585,17 +775,122 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   CUB(cudaMemcpyAsync(p, S.p_before, (size_t)B * N * sizeof(double), cudaMemcpyDeviceToHost, st));
   if(norm2x_out) CUB(cudaMemcpyAsync(norm2x_out, S.n2x_before, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost, st));
   if(iterations_out) CUB(cudaMemcpyAsync(iterations_out, S.steps, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
+  if(h)
+  {
+    CUB(cudaMemcpyAsync(h->JtJ, S.JtJ, (size_t)B * N * N * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    CUB(cudaMemcpyAsync(h->lambda, S.lambda, (size_t)B * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  }
   CUB(cudaStreamSynchronize(st));
   result = (int)B - *h_active;
+  if(h) { *returnBatch = h; h = 0; }
 fail:
+  if(h) batch_destroy(h);
   return result;
 }
 
-extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate, unsigned int Nmeas,
-                                                 unsigned int B, dogleg_gpu_callback_dense_batched_t* f,
-                                                 void* cookie, const dogleg_parameters2_t* parameters,
-                                                 double* norm2x_out, int* iterations_out)
+// enqueue k_batched_factor on st, after the handle's earlier work; it becomes the handle's latest
+static int batch_enqueue(dogleg_gpu_batch_t* h, const double* d_R, double* d_X, int nrhs, int packed, int* nfail,
+                         cudaStream_t st)
 {
+  typedef void (*factor_kernel_t)(BatchFactorArgs);
+  const int nt8 = (h->N + 7) / 8, ld = 8 * nt8 + 1;
+  const factor_kernel_t kern = nt8 == 1 ? k_batched_factor<1> : nt8 == 2 ? k_batched_factor<2>
+                             : nt8 == 3 ? k_batched_factor<3> : k_batched_factor<4>;
+  const size_t smem = sizeof(double) * (size_t)BT_WARPS * (32 * ld + 8 * nt8 * ld + 8 * nt8);
+  BatchFactorArgs A = { h->B, h->N, nrhs, h->JtJ, h->lambda, d_R, d_X, packed, nfail };
+  CUB(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  CUB(cudaStreamWaitEvent(st, h->ev, 0));
+  kern<<<(h->B + BT_WARPS - 1) / BT_WARPS, BT_NT, smem, st>>>(A);
+  CUB(cudaGetLastError());
+  CUB(cudaEventRecord(h->ev, st));
+  return 0;
+fail:
+  return -1;
+}
+
+// the host-pointer forms: stage through device buffers on the handle's stream; returns the failed problems
+static int batch_host(dogleg_gpu_batch_t* h, const double* R, double* X, int nrhs, int packed)
+{
+  DeviceScope ds(h->device);
+  const size_t nin = R ? (size_t)h->B * h->N * nrhs : 0;
+  const size_t nout = packed ? (size_t)h->B * (h->N * (h->N + 1) / 2) : (size_t)h->B * h->N * (R ? nrhs : h->N);
+  double *dR = 0, *dX = 0;
+  int nfail = 0, result = -1;
+  CUB(cudaMalloc((void**)&dX, nout * sizeof(double)));
+  if(R)
+  {
+    CUB(cudaMalloc((void**)&dR, nin * sizeof(double)));
+    CUB(cudaMemcpyAsync(dR, R, nin * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  }
+  CUB(cudaStreamWaitEvent(h->st, h->ev, 0));
+  CUB(cudaMemsetAsync(h->nfail, 0, sizeof(int), h->st));
+  if(batch_enqueue(h, dR, dX, nrhs, packed, h->nfail, h->st)) goto fail;
+  CUB(cudaMemcpyAsync(X, dX, nout * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaMemcpyAsync(&nfail, h->nfail, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaStreamSynchronize(h->st));
+  result = nfail;
+fail:
+  cudaFree(dR); cudaFree(dX);
+  return result;
+}
+
+extern "C" int dogleg_gpu_batch_status(const dogleg_gpu_batch_t* h, int* status_out, double* lambda_out)
+{
+  if(!h) { dlb_set_error("dogleg_gpu_batch_status: NULL handle"); return -1; }
+  DeviceScope ds(h->device);
+  CUB(cudaStreamWaitEvent(h->st, h->ev, 0));
+  if(status_out) CUB(cudaMemcpyAsync(status_out, h->status, (size_t)h->B * sizeof(int), cudaMemcpyDeviceToHost, h->st));
+  if(lambda_out) CUB(cudaMemcpyAsync(lambda_out, h->lambda, (size_t)h->B * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaStreamSynchronize(h->st));
+  return 0;
+fail:
+  return -1;
+}
+
+extern "C" int dogleg_gpu_batch_solve(dogleg_gpu_batch_t* h, const double* R, double* X, int nrhs)
+{
+  if(!h) { dlb_set_error("dogleg_gpu_batch_solve: NULL handle"); return -1; }
+  if(!R || !X || nrhs < 1) { dlb_set_error("dogleg_gpu_batch_solve: bad arguments (needs R, X and nrhs >= 1)"); return -1; }
+  return batch_host(h, R, X, nrhs, 0);
+}
+
+extern "C" int dogleg_gpu_batch_solve_device(dogleg_gpu_batch_t* h, const double* d_R, double* d_X, int nrhs, void* stream)
+{
+  if(!h) { dlb_set_error("dogleg_gpu_batch_solve_device: NULL handle"); return -1; }
+  if(!d_R || !d_X || nrhs < 1) { dlb_set_error("dogleg_gpu_batch_solve_device: bad arguments (needs d_R, d_X and nrhs >= 1)"); return -1; }
+  DeviceScope ds(h->device);
+  return batch_enqueue(h, d_R, d_X, nrhs, 0, 0, (cudaStream_t)stream);
+}
+
+extern "C" int dogleg_gpu_batch_covariance(dogleg_gpu_batch_t* h, double* out, int packed)
+{
+  if(!h) { dlb_set_error("dogleg_gpu_batch_covariance: NULL handle"); return -1; }
+  if(!out) { dlb_set_error("dogleg_gpu_batch_covariance: bad arguments (needs out)"); return -1; }
+  return batch_host(h, 0, out, h->N, packed != 0);
+}
+
+extern "C" int dogleg_gpu_batch_covariance_device(dogleg_gpu_batch_t* h, double* d_out, int packed, void* stream)
+{
+  if(!h) { dlb_set_error("dogleg_gpu_batch_covariance_device: NULL handle"); return -1; }
+  if(!d_out) { dlb_set_error("dogleg_gpu_batch_covariance_device: bad arguments (needs d_out)"); return -1; }
+  DeviceScope ds(h->device);
+  return batch_enqueue(h, 0, d_out, h->N, packed != 0, 0, (cudaStream_t)stream);
+}
+
+extern "C" void dogleg_gpu_batch_free(dogleg_gpu_batch_t** batch)
+{
+  if(!batch || !*batch) return;
+  batch_destroy(*batch);
+  *batch = 0;
+}
+
+extern "C" int dogleg_gpu_optimize_dense_batched2(double* p, unsigned int Nstate, unsigned int Nmeas,
+                                                  unsigned int B, dogleg_gpu_callback_dense_batched_t* f,
+                                                  void* cookie, const dogleg_parameters2_t* parameters,
+                                                  double* norm2x_out, int* iterations_out,
+                                                  dogleg_gpu_batch_t** returnBatch)
+{
+  if(returnBatch) *returnBatch = 0;
   if(dogleg_gpu_device_count() <= 0) { dlb_set_error("no CUDA device available: libdogleg-b200 has no CPU fallback"); return -1; }
   if(!f || !p || B == 0) { dlb_set_error("dense_batched: bad arguments"); return -1; }
   const int N = (int)Nstate;
@@ -604,14 +899,25 @@ extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate,
     dlb_set_error("dense_batched: needs Nstate <= 32; use dogleg_optimize_dense2 per problem for bigger ones");
     return -1;
   }
-  return batched_solve(BF_DENSE, p, N, (int)Nmeas, B, (void*)f, cookie, parameters, norm2x_out, iterations_out);
+  return batched_solve(BF_DENSE, p, N, (int)Nmeas, B, (void*)f, cookie, parameters, norm2x_out, iterations_out,
+                       returnBatch);
 }
 
-extern "C" int dogleg_gpu_optimize_dense_products_batched(double* p, unsigned int Nstate, unsigned int B,
-                                                          dogleg_gpu_callback_dense_products_batched_t* f, void* cookie,
-                                                          const dogleg_parameters2_t* parameters,
-                                                          double* norm2x_out, int* iterations_out)
+extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate, unsigned int Nmeas,
+                                                 unsigned int B, dogleg_gpu_callback_dense_batched_t* f,
+                                                 void* cookie, const dogleg_parameters2_t* parameters,
+                                                 double* norm2x_out, int* iterations_out)
 {
+  return dogleg_gpu_optimize_dense_batched2(p, Nstate, Nmeas, B, f, cookie, parameters, norm2x_out, iterations_out, 0);
+}
+
+extern "C" int dogleg_gpu_optimize_dense_products_batched2(double* p, unsigned int Nstate, unsigned int B,
+                                                           dogleg_gpu_callback_dense_products_batched_t* f, void* cookie,
+                                                           const dogleg_parameters2_t* parameters,
+                                                           double* norm2x_out, int* iterations_out,
+                                                           dogleg_gpu_batch_t** returnBatch)
+{
+  if(returnBatch) *returnBatch = 0;
   if(dogleg_gpu_device_count() <= 0) { dlb_set_error("no CUDA device available: libdogleg-b200 has no CPU fallback"); return -1; }
   if(!f || !p || B == 0) { dlb_set_error("dense_products_batched: bad arguments (needs p, a callback and B > 0)"); return -1; }
   const int N = (int)Nstate;
@@ -627,5 +933,13 @@ extern "C" int dogleg_gpu_optimize_dense_products_batched(double* p, unsigned in
     return -1;
   }
   return batched_solve(packed ? BF_PRODUCTS_PACKED : BF_PRODUCTS_FULL, p, N, 0, B, (void*)f, cookie, parameters,
-                       norm2x_out, iterations_out);
+                       norm2x_out, iterations_out, returnBatch);
+}
+
+extern "C" int dogleg_gpu_optimize_dense_products_batched(double* p, unsigned int Nstate, unsigned int B,
+                                                          dogleg_gpu_callback_dense_products_batched_t* f, void* cookie,
+                                                          const dogleg_parameters2_t* parameters,
+                                                          double* norm2x_out, int* iterations_out)
+{
+  return dogleg_gpu_optimize_dense_products_batched2(p, Nstate, B, f, cookie, parameters, norm2x_out, iterations_out, 0);
 }

@@ -10,6 +10,8 @@ SOLVE_DENSE, SOLVE_SPARSE, SOLVE_DENSE_PRODUCTS = 0, 1, 2      # dogleg_solve_ty
 DEBUG_VNLOG = 1 << 30
 BUF_P, BUF_X, BUF_JTX, BUF_CAUCHY, BUF_GN, BUF_STEP, BUF_JVALUES, BUF_JP, BUF_JI, BUF_NORM2X = range(10)
 STEP_CAUCHY, STEP_GAUSSNEWTON, STEP_INTERPOLATED = 0, 1, 2
+# DOGLEG_GPU_BATCH_*: why a problem of a batched solve stopped (dogleg_gpu_batch_status)
+BATCH_UNFINISHED, BATCH_GRADIENT, BATCH_STEP, BATCH_TRUSTREGION, BATCH_MAX_ITERATIONS = range(5)
 SYM = dict(perm=0, parent=1, colcount=2, sn_first=3, rows_ptr=4, rows=5, sn_parent=6,
            cls_of_col=7, cls_front=8, sn_level=9, rel=10, child_ptr=11, child_list=12, level_ptr=13,
            level_sn=14, cls_ptr=15, cls_rows=16, cls_loc=17, mem_ptr=18, mem_col=19)
@@ -116,6 +118,22 @@ def load():
     L.dogleg_gpu_optimize_dense_products.restype = C.c_double
     L.dogleg_gpu_optimize_dense_products_batched.argtypes = [dp, C.c_uint, C.c_uint, vp, vp, PP, dp, ip]
     L.dogleg_gpu_optimize_dense_products_batched.restype = C.c_int
+    L.dogleg_gpu_optimize_dense_batched2.argtypes = [dp, C.c_uint, C.c_uint, C.c_uint, vp, vp, PP, dp, ip, C.POINTER(vp)]
+    L.dogleg_gpu_optimize_dense_batched2.restype = C.c_int
+    L.dogleg_gpu_optimize_dense_products_batched2.argtypes = [dp, C.c_uint, C.c_uint, vp, vp, PP, dp, ip, C.POINTER(vp)]
+    L.dogleg_gpu_optimize_dense_products_batched2.restype = C.c_int
+    L.dogleg_gpu_batch_status.argtypes = [vp, ip, dp]
+    L.dogleg_gpu_batch_status.restype = C.c_int
+    L.dogleg_gpu_batch_solve.argtypes = [vp, dp, dp, C.c_int]
+    L.dogleg_gpu_batch_solve.restype = C.c_int
+    L.dogleg_gpu_batch_solve_device.argtypes = [vp, vp, vp, C.c_int, vp]
+    L.dogleg_gpu_batch_solve_device.restype = C.c_int
+    L.dogleg_gpu_batch_covariance.argtypes = [vp, dp, C.c_int]
+    L.dogleg_gpu_batch_covariance.restype = C.c_int
+    L.dogleg_gpu_batch_covariance_device.argtypes = [vp, vp, C.c_int, vp]
+    L.dogleg_gpu_batch_covariance_device.restype = C.c_int
+    L.dogleg_gpu_batch_free.argtypes = [C.POINTER(vp)]
+    L.dogleg_gpu_batch_free.restype = None
     L.dogleg_gpu_release_batched_cache.restype = None
     L.dogleg_gpu_batched_stats.argtypes = [dp]
     L.dogleg_gpu_batched_stats.restype = None
