@@ -223,6 +223,21 @@ int  dogleg_gpu_batch_solve_device(dogleg_gpu_batch_t* batch, const double* d_R,
  * the upper triangle of that row-first matrix, packed row-first (the products layout) */
 int  dogleg_gpu_batch_covariance(dogleg_gpu_batch_t* batch, double* out, int packed);
 int  dogleg_gpu_batch_covariance_device(dogleg_gpu_batch_t* batch, double* d_out, int packed, void* stream);
+/* dogleg_getOutliernessFactors() for every problem of a batch (reference dogleg.c:2294-2399, 2401-2791), on
+ * JtJ_b + lambda_b I of the handle (the matrix of dogleg_gpu_batch_covariance; the ladder may raise lambda_b and
+ * stores it, as there). x: B x Nmeas and J: B x Nmeas x Nstate (row-first per problem), both evaluated by the
+ * caller at the p the solve returned. Feature f of a problem = measurements [f*featureSize, (f+1)*featureSize);
+ * featureSize 1 or 2 (<= 1 means 1, as in the reference). factors: B x Nfeatures. scale: B, in/out: entries > 0
+ * are kept, the others are set from |x_b|^2, Nmeas and NoutlierFeatures[b] as the reference does.
+ * NoutlierFeatures: B entries or NULL (all 0). Works on handles of either batched form. Return values as
+ * dogleg_gpu_batch_solve / _solve_device (host form: number of problems whose factors are NaN). */
+int  dogleg_gpu_batch_outlierness(dogleg_gpu_batch_t* batch, const double* x, const double* J, unsigned int Nmeas,
+                                  int featureSize, int Nfeatures, const int* NoutlierFeatures,
+                                  double* scale, double* factors);
+int  dogleg_gpu_batch_outlierness_device(dogleg_gpu_batch_t* batch, const double* d_x, const double* d_J,
+                                         unsigned int Nmeas, int featureSize, int Nfeatures,
+                                         const int* d_NoutlierFeatures, double* d_scale, double* d_factors,
+                                         void* stream);
 void dogleg_gpu_batch_free(dogleg_gpu_batch_t** batch);   /* sets *batch = NULL; NULL is fine */
 
 /* statistics of this thread's last batched solve (either form): [0] trial launches, [1] sum over launches of

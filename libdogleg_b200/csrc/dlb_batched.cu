@@ -27,13 +27,16 @@
 //
 // Final state (the `2` entry points with a dogleg_gpu_batch_t): the trial kernel also keeps the final point's
 // JtJ and writes why each problem stopped; k_batched_factor factors every problem's JtJ + lambda I with the
-// same ladder and solves with it (dogleg_gpu_batch_solve, dogleg_gpu_batch_covariance).
+// same ladder and solves with it (dogleg_gpu_batch_solve, dogleg_gpu_batch_covariance); k_batched_outlierness
+// computes every problem's outlierness factors on the same matrix (dogleg_gpu_batch_outlierness).
 #include "dlb_common.cuh"
 #include "dogleg_gpu.h"
+#include "dlb_outlier_math.h"
 #include <vector>
 #include <cstring>
 #include <string>
 #include <algorithm>
+#include <climits>
 
 extern "C" void dlb_set_error(const char* msg);
 
@@ -457,6 +460,42 @@ k_batched_trial(BatchState S)
 }
 
 // ---- solves with the final state of a batched solve (dogleg_gpu_batch_t) ----
+// The warp's problem JtJ (N x N row-first, global) + lambda I factored by the trial kernel's ladder, starting from
+// the lambda at *glam: JtJ is staged in sY (row stride 8 * NT8 + 1), L goes to sL and the reciprocal pivots to srs.
+// Returns the lambda taken (not finite: no lambda of the ladder gave a positive definite matrix).
+template<int NT8>
+__device__ __forceinline__ double bt_load_and_factor(const double* gA, const double* glam, double* sY, double* sL,
+                                                     double* srs, int N, int lane)
+{
+  constexpr int NMAX = 8 * NT8, LD = NMAX + 1;
+  for(int e = lane; e < N * N; e += 32) { const int a = e / N, c = e - a * N; sY[a * LD + c] = ldg_stream(gA + e); }
+  double lam = *glam;
+  __syncwarp();
+  double Lr[NMAX], rsv[NMAX];
+  bt_cholesky_ladder<NT8>(sY, sL, N, lane, lam, Lr, rsv);
+#pragma unroll
+  for(int j = 0; j < NMAX; j++)
+    if(j < N && lane == j) srs[j] = rsv[j];
+  return lam;
+}
+
+// L y = r in place for this lane's right-hand side y (entries >= N are never read); L and the reciprocal pivots
+// from the warp's shared memory, every lane reading the same entry (broadcasts)
+template<int NT8>
+__device__ __forceinline__ void bt_forward_subst(const double* sL, const double* srs, int N, double (&y)[8 * NT8])
+{
+  constexpr int NMAX = 8 * NT8, LD = NMAX + 1;
+#pragma unroll
+  for(int j = 0; j < NMAX; j++)
+  {
+    if(j >= N) continue;
+    double acc = y[j];
+#pragma unroll
+    for(int i = 0; i < j; i++) acc = fma(-sL[j * LD + i], y[i], acc);
+    y[j] = acc * srs[j];
+  }
+}
+
 struct BatchFactorArgs
 {
   int B, N, nrhs;             // nrhs: columns of R and X
@@ -486,17 +525,7 @@ __global__ void __launch_bounds__(BT_NT) k_batched_factor(BatchFactorArgs A)
   double* sY  = sm + (size_t)w * (32 * LD + NMAX * LD + NMAX);   // JtJ, then right-hand sides / results
   double* sL  = sY + 32 * LD;                                     // Cholesky factor
   double* srs = sL + NMAX * LD;                                   // reciprocal pivots
-  const double* gA = A.JtJ + (size_t)b * N * N;
-  for(int e = lane; e < N * N; e += 32) { const int a = e / N, c = e - a * N; sY[a * LD + c] = ldg_stream(gA + e); }
-  double lam = A.lambda[b];
-  __syncwarp();
-  {
-    double Lr[NMAX], rsv[NMAX];
-    bt_cholesky_ladder<NT8>(sY, sL, N, lane, lam, Lr, rsv);
-#pragma unroll
-    for(int j = 0; j < NMAX; j++)
-      if(j < N && lane == j) srs[j] = rsv[j];
-  }
+  const double lam = bt_load_and_factor<NT8>(A.JtJ + (size_t)b * N * N, A.lambda + b, sY, sL, srs, N, lane);
   const bool failed = !isfinite(lam);
   if(lane == 0) { A.lambda[b] = lam; if(failed && A.nfail) atomicAdd(A.nfail, 1); }
   __syncwarp();
@@ -515,15 +544,7 @@ __global__ void __launch_bounds__(BT_NT) k_batched_factor(BatchFactorArgs A)
     double y[NMAX];                                               // entries >= N are never read
 #pragma unroll
     for(int i = 0; i < NMAX; i++) y[i] = gR ? sY[lane * LD + i] : (i == c0 + lane ? 1.0 : 0.0);
-#pragma unroll
-    for(int j = 0; j < NMAX; j++)                                 // L y = r
-    {
-      if(j >= N) continue;
-      double acc = y[j];
-#pragma unroll
-      for(int i = 0; i < j; i++) acc = fma(-sL[j * LD + i], y[i], acc);
-      y[j] = acc * srs[j];
-    }
+    bt_forward_subst<NT8>(sL, srs, N, y);                        // L y = r
 #pragma unroll
     for(int j = NMAX - 1; j >= 0; j--)                            // L' x = y
     {
@@ -551,6 +572,100 @@ __global__ void __launch_bounds__(BT_NT) k_batched_factor(BatchFactorArgs A)
     else
       for(int e = lane; e < nc * N; e += 32) { const int k = e / N, i = e - k * N; gX[(size_t)c0 * N + e] = sY[k * LD + i]; }
     __syncwarp();
+  }
+}
+
+// ---- outlierness factors of every problem (dogleg_gpu_batch_outlierness) ----
+struct BatchOutlierArgs
+{
+  int B, N, M, fsize, nfeat;  // M: measurements per problem; features are fsize consecutive ones, nfeat * fsize <= M
+  const double* JtJ;          // B x N*N
+  double* lambda;             // B; raised in place by the ladder
+  const double* x;            // B x M
+  const double* J;            // B x M x N, row-first per problem
+  const int* nout;            // B NoutlierFeatures, or NULL (all 0)
+  double* scale;              // B, in / out
+  double* factors;            // B x nfeat
+  int* nfail;
+};
+
+// One warp per problem. A_ij of a feature is j_i' inv(JtJ + lambda I) j_j = (L^-1 j_i) . (L^-1 j_j), so one forward
+// substitution per measurement is all it takes. J is taken 32 rows at a time: a problem's row-first M x N block has
+// the layout of k_batched_factor's column-major N x M right-hand sides, and is staged through shared memory the same
+// way (coalesced reads); then lane == measurement substitutes its row against the broadcast L. The next chunk's
+// loads are in flight during the current chunk's substitution. |x|^2 is a fixed-order warp sum and A_01 of a pair
+// takes the neighbouring lane's row by shuffles, so the factors are reproducible bit for bit.
+template<int NT8>
+__global__ void __launch_bounds__(BT_NT) k_batched_outlierness(BatchOutlierArgs A)
+{
+  extern __shared__ double sm[];
+  constexpr int NMAX = 8 * NT8, LD = NMAX + 1;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int b = blockIdx.x * BT_WARPS + w;
+  if(b >= A.B) return;
+  const int N = A.N, M = A.M, fs = A.fsize;
+  double* sY  = sm + (size_t)w * (32 * LD + NMAX * LD + NMAX);   // JtJ, then rows of J
+  double* sL  = sY + 32 * LD;
+  double* srs = sL + NMAX * LD;
+  const double lam = bt_load_and_factor<NT8>(A.JtJ + (size_t)b * N * N, A.lambda + b, sY, sL, srs, N, lane);
+  const bool failed = !isfinite(lam);
+  if(lane == 0) { A.lambda[b] = lam; if(failed && A.nfail) atomicAdd(A.nfail, 1); }
+
+  const double* gx = A.x + (size_t)b * M;
+  const double* gJ = A.J + (size_t)b * M * N;
+  double n2 = 0.0;
+  for(int m = lane; m < M; m += 32) { const double v = ldg_stream(gx + m); n2 = fma(v, v, n2); }
+  double k = A.scale[b];
+  outlierness_scale(&k, M, N, A.nout ? A.nout[b] : 0, fs, warp_sum_all(n2));
+  if(lane == 0) A.scale[b] = k;
+
+  // this lane's share of the 32-row chunk at row m0: entries lane + 32 t of the chunk's min(32, M - m0) * N
+  double v[NMAX];
+  auto load_chunk = [&](int m0) {
+    const int ne = min(32, M - m0) * N;
+#pragma unroll
+    for(int t = 0; t < NMAX; t++)
+      if(t < N && lane + 32 * t < ne) v[t] = ldg_stream(gJ + (size_t)m0 * N + lane + 32 * t);
+  };
+  const int Mused = A.nfeat * fs;
+  double* gf = A.factors + (size_t)b * A.nfeat;
+  load_chunk(0);
+  for(int m0 = 0; m0 < Mused; m0 += 32)
+  {
+    const int ne = min(32, M - m0) * N;
+    __syncwarp();
+#pragma unroll
+    for(int t = 0; t < NMAX; t++)
+      if(t < N && lane + 32 * t < ne) { const int e = lane + 32 * t, r = e / N; sY[r * LD + e - r * N] = v[t]; }
+    __syncwarp();
+    double y[NMAX];                                               // entries >= N are never read
+#pragma unroll
+    for(int i = 0; i < NMAX; i++) y[i] = sY[lane * LD + i];
+    const int m = m0 + lane;
+    const double xm = m < M ? ldg_stream(gx + m) : 0.0;
+    if(m0 + 32 < Mused) load_chunk(m0 + 32);
+    bt_forward_subst<NT8>(sL, srs, N, y);
+    double a = 0.0, a01 = 0.0;
+#pragma unroll
+    for(int i = 0; i < NMAX; i++)
+      if(i < N)
+      {
+        a = fma(y[i], y[i], a);
+        if(fs == 2) a01 = fma(y[i], __shfl_down_sync(0xffffffffu, y[i], 1), a01);
+      }
+    double f;
+    if(fs == 1)
+    {
+      outlierness_factor(&f, &xm, &a, 1, k);
+      if(m < Mused) gf[m] = failed ? __longlong_as_double(0x7ff8000000000000LL) : f;
+    }
+    else
+    {
+      const double A2[3] = { a, a01, __shfl_down_sync(0xffffffffu, a, 1) };
+      const double x2[2] = { xm, __shfl_down_sync(0xffffffffu, xm, 1) };
+      outlierness_factor(&f, x2, A2, 2, k);
+      if(!(lane & 1) && m < Mused) gf[m >> 1] = failed ? __longlong_as_double(0x7ff8000000000000LL) : f;
+    }
   }
 }
 
@@ -875,6 +990,91 @@ extern "C" int dogleg_gpu_batch_covariance_device(dogleg_gpu_batch_t* h, double*
   if(!d_out) { dlb_set_error("dogleg_gpu_batch_covariance_device: bad arguments (needs d_out)"); return -1; }
   DeviceScope ds(h->device);
   return batch_enqueue(h, 0, d_out, h->N, packed != 0, 0, (cudaStream_t)stream);
+}
+
+// the argument checks of both outlierness calls; featureSize <= 1 means 1 (as in the reference)
+static bool outlier_args_ok(const char* fn, const dogleg_gpu_batch_t* h, const void* x, const void* J, const void* scale,
+                            const void* factors, unsigned int Nmeas, int& featureSize, int Nfeatures)
+{
+  std::string msg;
+  if(featureSize <= 1) featureSize = 1;
+  if(!h) msg = "NULL handle";
+  else if(!x || !J || !scale || !factors) msg = "bad arguments (needs x, J, scale and factors)";
+  else if(featureSize > 2) msg = "featureSize > 2 not implemented yet. Got featureSize=" + std::to_string(featureSize);
+  else if(Nfeatures < 1 || Nmeas < 1 || Nmeas > (unsigned int)INT_MAX) msg = "bad arguments (needs Nfeatures >= 1 and Nmeas >= 1)";
+  else if((long long)Nfeatures * featureSize > (long long)Nmeas) msg = "Nfeatures*featureSize exceeds Nmeas";
+  if(msg.empty()) return true;
+  dlb_set_error((std::string(fn) + ": " + msg).c_str());
+  return false;
+}
+
+// enqueue k_batched_outlierness on st, after the handle's earlier work; it becomes the handle's latest
+static int batch_outlier_enqueue(dogleg_gpu_batch_t* h, const double* d_x, const double* d_J, int M, int fsize,
+                                 int nfeat, const int* d_nout, double* d_scale, double* d_factors, int* nfail,
+                                 cudaStream_t st)
+{
+  typedef void (*outlier_kernel_t)(BatchOutlierArgs);
+  const int nt8 = (h->N + 7) / 8, ld = 8 * nt8 + 1;
+  const outlier_kernel_t kern = nt8 == 1 ? k_batched_outlierness<1> : nt8 == 2 ? k_batched_outlierness<2>
+                              : nt8 == 3 ? k_batched_outlierness<3> : k_batched_outlierness<4>;
+  const size_t smem = sizeof(double) * (size_t)BT_WARPS * (32 * ld + 8 * nt8 * ld + 8 * nt8);
+  BatchOutlierArgs A = { h->B, h->N, M, fsize, nfeat, h->JtJ, h->lambda, d_x, d_J, d_nout, d_scale, d_factors, nfail };
+  CUB(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  CUB(cudaStreamWaitEvent(st, h->ev, 0));
+  kern<<<(h->B + BT_WARPS - 1) / BT_WARPS, BT_NT, smem, st>>>(A);
+  CUB(cudaGetLastError());
+  CUB(cudaEventRecord(h->ev, st));
+  return 0;
+fail:
+  return -1;
+}
+
+extern "C" int dogleg_gpu_batch_outlierness(dogleg_gpu_batch_t* h, const double* x, const double* J, unsigned int Nmeas,
+                                            int featureSize, int Nfeatures, const int* NoutlierFeatures,
+                                            double* scale, double* factors)
+{
+  if(!outlier_args_ok("dogleg_gpu_batch_outlierness", h, x, J, scale, factors, Nmeas, featureSize, Nfeatures)) return -1;
+  DeviceScope ds(h->device);
+  const size_t B = (size_t)h->B, nx = B * Nmeas, nJ = nx * h->N, nf = B * Nfeatures;
+  double *dx = 0, *dJ = 0, *dscale = 0, *df = 0;
+  int* dnout = 0;
+  int nfail = 0, result = -1;
+  CUB(cudaMalloc((void**)&dx, nx * sizeof(double)));
+  CUB(cudaMalloc((void**)&dJ, nJ * sizeof(double)));
+  CUB(cudaMalloc((void**)&dscale, B * sizeof(double)));
+  CUB(cudaMalloc((void**)&df, nf * sizeof(double)));
+  CUB(cudaMemcpyAsync(dx, x, nx * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  CUB(cudaMemcpyAsync(dJ, J, nJ * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  CUB(cudaMemcpyAsync(dscale, scale, B * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  if(NoutlierFeatures)
+  {
+    CUB(cudaMalloc((void**)&dnout, B * sizeof(int)));
+    CUB(cudaMemcpyAsync(dnout, NoutlierFeatures, B * sizeof(int), cudaMemcpyHostToDevice, h->st));
+  }
+  CUB(cudaStreamWaitEvent(h->st, h->ev, 0));
+  CUB(cudaMemsetAsync(h->nfail, 0, sizeof(int), h->st));
+  if(batch_outlier_enqueue(h, dx, dJ, (int)Nmeas, featureSize, Nfeatures, dnout, dscale, df, h->nfail, h->st)) goto fail;
+  CUB(cudaMemcpyAsync(factors, df, nf * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaMemcpyAsync(scale, dscale, B * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaMemcpyAsync(&nfail, h->nfail, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaStreamSynchronize(h->st));
+  result = nfail;
+fail:
+  cudaFree(dx); cudaFree(dJ); cudaFree(dscale); cudaFree(df); cudaFree(dnout);
+  return result;
+}
+
+extern "C" int dogleg_gpu_batch_outlierness_device(dogleg_gpu_batch_t* h, const double* d_x, const double* d_J,
+                                                   unsigned int Nmeas, int featureSize, int Nfeatures,
+                                                   const int* d_NoutlierFeatures, double* d_scale, double* d_factors,
+                                                   void* stream)
+{
+  if(!outlier_args_ok("dogleg_gpu_batch_outlierness_device", h, d_x, d_J, d_scale, d_factors, Nmeas, featureSize,
+                      Nfeatures))
+    return -1;
+  DeviceScope ds(h->device);
+  return batch_outlier_enqueue(h, d_x, d_J, (int)Nmeas, featureSize, Nfeatures, d_NoutlierFeatures, d_scale, d_factors,
+                               0, (cudaStream_t)stream);
 }
 
 extern "C" void dogleg_gpu_batch_free(dogleg_gpu_batch_t** batch)

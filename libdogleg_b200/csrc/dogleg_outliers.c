@@ -26,49 +26,12 @@
 #include "dogleg.h"
 #include "dogleg_gpu.h"
 #include "dogleg_internal.h"
+#include "dlb_outlier_math.h"
 
 #define SAY(fmt, ...) fprintf(stderr, "libdogleg at %s:%d: " fmt "\n", __FILE__, __LINE__, ## __VA_ARGS__)
 #define SAY_IF_VERBOSE(fmt, ...) do { if(ctx->parameters->debug && !ctx->parameters->debug_vnlog) SAY(fmt, ## __VA_ARGS__); } while(0)
 #define OUTLIER_CHUNK 64
 #define OUTLIER_CONFIDENCE_DROP_THRESHOLD 0.05
-
-/* k = N_ok / (4 (Nstate+1) |x|^2 / (N_ok - Nstate - 1)), kept if already positive (dogleg.c:2381-2399) */
-static void outlierness_scale(double* scale, int Nmeasurements, int Nstate, int NoutlierFeatures,
-                              int featureSize, double norm2_x)
-{
-  if(*scale > 0.0) return;
-  const int Nok = Nmeasurements - NoutlierFeatures * featureSize;
-  *scale = (double)Nok / (4. * ((double)(Nstate + 1) * norm2_x / (double)(Nok - Nstate - 1)));
-}
-
-/* A holds the upper triangle row-first: [a00] or [a00 a01 a11] (dogleg.c:2294-2379) */
-static bool outlierness_factor(double* factor, const double* x, const double* A, int featureSize, double k)
-{
-  if(featureSize == 1)
-  {
-    const double denom = 1.0 - A[0];
-    if(fabs(denom) < 1e-8) { *factor = DBL_MAX; return true; }      /* certainly an outlier */
-    *factor = x[0] * x[0] / denom;
-  }
-  else if(featureSize == 2)
-  {
-    const double det = (1.0 - A[0]) * (1.0 - A[2]) - A[1] * A[1];
-    if(fabs(det) < 1e-8) { *factor = DBL_MAX; return true; }
-    /* B = inv(A - I) scaled by det; Cook's self+others: x'Bx + |Bx|^2 */
-    const double B00 = A[2] - 1.0, B11 = A[0] - 1.0, B01 = -A[1];
-    const double xBx = (x[0] * x[0] * B00 + x[0] * x[1] * B01 * 2.0 + x[1] * x[1] * B11) / det;
-    const double v1 = x[0] * B00 + x[1] * B01, v2 = x[0] * B01 + x[1] * B11;
-    *factor = xBx + (v1 * v1 + v2 * v2) / (det * det);
-  }
-  else
-  {
-    SAY("featureSize > 2 not implemented yet. Got featureSize=%d", featureSize);
-    return false;
-  }
-  /* the reference's own "hack": the threshold should be 1 but the scale is divided by 8 (dogleg.c:2373-2375) */
-  *factor *= k / 8.;
-  return true;
-}
 
 bool dogleg_getOutliernessFactors(double* factors, double* scale, int featureSize, int Nfeatures,
                                   int NoutlierFeatures, dogleg_operatingPoint_t* point, dogleg_solverContext_t* ctx)

@@ -132,6 +132,10 @@ def load():
     L.dogleg_gpu_batch_covariance.restype = C.c_int
     L.dogleg_gpu_batch_covariance_device.argtypes = [vp, vp, C.c_int, vp]
     L.dogleg_gpu_batch_covariance_device.restype = C.c_int
+    L.dogleg_gpu_batch_outlierness.argtypes = [vp, dp, dp, C.c_uint, C.c_int, C.c_int, ip, dp, dp]
+    L.dogleg_gpu_batch_outlierness.restype = C.c_int
+    L.dogleg_gpu_batch_outlierness_device.argtypes = [vp, vp, vp, C.c_uint, C.c_int, C.c_int, vp, vp, vp, vp]
+    L.dogleg_gpu_batch_outlierness_device.restype = C.c_int
     L.dogleg_gpu_batch_free.argtypes = [C.POINTER(vp)]
     L.dogleg_gpu_batch_free.restype = None
     L.dogleg_gpu_release_batched_cache.restype = None
