@@ -193,6 +193,26 @@ int dogleg_gpu_optimize_dense_products_batched2(double* p, unsigned int Nstate, 
                                                 double* norm2x_out, int* iterations_out,
                                                 dogleg_gpu_batch_t** returnBatch);
 
+/* Batched dense problems with different numbers of measurements, stored without padding. Problem b has Nmeas[b]
+ * measurements (Nmeas: host, B entries); its residuals are at d_x + d_row_off[b] and its Nmeas[b] x Nstate
+ * Jacobian (row-first) at d_J + d_row_off[b] * Nstate, where d_row_off (device, B + 1 entries, 64-bit) holds the
+ * exclusive prefix sums of Nmeas. Nmeas[b] == 0 is allowed (the problem stops at its start point with
+ * DOGLEG_GPU_BATCH_GRADIENT), and so is Nmeas[b] < Nstate (a singular JtJ: the lambda ladder handles it). The
+ * results are those of dogleg_gpu_optimize_dense_batched2 on the batch zero-padded to its longest problem, bit for
+ * bit. p, norm2x_out, iterations_out, returnBatch, d_active and the return value as there; Nstate <= 32. Refused
+ * before the first callback: Nstate outside 1..32, B == 0, a NULL p, Nmeas or callback, a count above INT_MAX and
+ * a batch that does not fit in device memory. */
+typedef void (dogleg_gpu_callback_dense_ragged_t)(const double* d_p, double* d_x, double* d_J,
+                                                  const long long* d_row_off, const int* d_active, int B,
+                                                  void* stream, void* cookie);
+int dogleg_gpu_optimize_dense_batched_ragged(double* p, unsigned int Nstate, const unsigned int* Nmeas,
+                                             unsigned int B, dogleg_gpu_callback_dense_ragged_t* f, void* cookie,
+                                             const dogleg_parameters2_t* parameters, double* norm2x_out,
+                                             int* iterations_out, dogleg_gpu_batch_t** returnBatch);
+/* the host side of a ragged solve: row_off (B + 1) = the prefix sums of Nmeas, order (B) = the problems longest
+ * first, ties by index (the order in which the trial kernel's warps take them). -1 if a count exceeds INT_MAX. */
+int dlb_batched_ragged_layout(const unsigned int* Nmeas, unsigned int B, long long* row_off, int* order);
+
 /* Why a problem stopped, in the order the single-problem solver tests (dogleg_core.c run_solver): after an
  * accepted step the gradient test comes before the iteration cap; at the initial point a problem is
  * GRADIENT if it has converged, else MAX_ITERATIONS if max_iterations <= 0. */
@@ -229,8 +249,9 @@ int  dogleg_gpu_batch_covariance_device(dogleg_gpu_batch_t* batch, double* d_out
  * caller at the p the solve returned. Feature f of a problem = measurements [f*featureSize, (f+1)*featureSize);
  * featureSize 1 or 2 (<= 1 means 1, as in the reference). factors: B x Nfeatures. scale: B, in/out: entries > 0
  * are kept, the others are set from |x_b|^2, Nmeas and NoutlierFeatures[b] as the reference does.
- * NoutlierFeatures: B entries or NULL (all 0). Works on handles of either batched form. Return values as
- * dogleg_gpu_batch_solve / _solve_device (host form: number of problems whose factors are NaN). */
+ * NoutlierFeatures: B entries or NULL (all 0). Works on handles of either uniform batched form; a handle from a
+ * ragged solve is refused. Return values as dogleg_gpu_batch_solve / _solve_device (host form: number of problems
+ * whose factors are NaN). */
 int  dogleg_gpu_batch_outlierness(dogleg_gpu_batch_t* batch, const double* x, const double* J, unsigned int Nmeas,
                                   int featureSize, int Nfeatures, const int* NoutlierFeatures,
                                   double* scale, double* factors);
@@ -238,6 +259,20 @@ int  dogleg_gpu_batch_outlierness_device(dogleg_gpu_batch_t* batch, const double
                                          unsigned int Nmeas, int featureSize, int Nfeatures,
                                          const int* d_NoutlierFeatures, double* d_scale, double* d_factors,
                                          void* stream);
+/* The same on a handle from dogleg_gpu_optimize_dense_batched_ragged (other handles are refused). x and J in the
+ * solve's layout: problem b's rows from row_off[b], the prefix sums of its Nmeas. factors is laid out like x:
+ * feature f of problem b goes to factors[row_off[b] + f]; the other entries are not written. Nfeatures: B counts,
+ * or NULL for Nmeas[b] / featureSize; fewer leave trailing rows (regularisation rows, say) out of the features,
+ * while the scale counts all of the problem's Nmeas[b] measurements. The host form refuses Nfeatures[b] < 0 or
+ * Nfeatures[b] * featureSize > Nmeas[b] before any work; the device form cannot check its device arrays, and such a
+ * problem gets a NaN scale and no factors. */
+int  dogleg_gpu_batch_outlierness_ragged(dogleg_gpu_batch_t* batch, const double* x, const double* J, int featureSize,
+                                         const int* Nfeatures, const int* NoutlierFeatures, double* scale,
+                                         double* factors);
+int  dogleg_gpu_batch_outlierness_ragged_device(dogleg_gpu_batch_t* batch, const double* d_x, const double* d_J,
+                                                int featureSize, const int* d_Nfeatures,
+                                                const int* d_NoutlierFeatures, double* d_scale, double* d_factors,
+                                                void* stream);
 void dogleg_gpu_batch_free(dogleg_gpu_batch_t** batch);   /* sets *batch = NULL; NULL is fine */
 
 /* statistics of this thread's last batched solve (either form): [0] trial launches, [1] sum over launches of

@@ -29,6 +29,10 @@
 // JtJ and writes why each problem stopped; k_batched_factor factors every problem's JtJ + lambda I with the
 // same ladder and solves with it (dogleg_gpu_batch_solve, dogleg_gpu_batch_covariance); k_batched_outlierness
 // computes every problem's outlierness factors on the same matrix (dogleg_gpu_batch_outlierness).
+//
+// Ragged form (dogleg_gpu_optimize_dense_batched_ragged): problem b has its own number of measurements, its rows
+// at row_off[b] of x and J. The RAGGED instantiations of the same two kernels take each warp's M and row pointers
+// from the offsets and its problem from a longest-first order; everything else is the uniform code.
 #include "dlb_common.cuh"
 #include "dogleg_gpu.h"
 #include "dlb_outlier_math.h"
@@ -37,6 +41,7 @@
 #include <string>
 #include <algorithm>
 #include <climits>
+#include <cstdint>
 
 extern "C" void dlb_set_error(const char* msg);
 
@@ -65,6 +70,10 @@ struct BatchState
   // a dogleg_gpu_batch_t was asked for (appended likewise): B termination codes (DOGLEG_GPU_BATCH_*), and the
   // final point's JtJ is kept in JtJ. NULL: neither.
   int *status;
+  // ragged form (appended likewise, read by the RAGGED instantiations only): problem b's rows are
+  // [row_off[b], row_off[b + 1]) of x and J; warp slot s takes problem order[s], longest first
+  const long long *row_off;
+  const int *order;
 };
 enum { FL_CAUCHY = 1, FL_GN = 2, FL_EDGE = 4, FL_PENDING = 8 };
 
@@ -151,15 +160,17 @@ __device__ __forceinline__ void bt_cholesky_ladder(const double* sA, double* sL,
 // products form at NT8 == 2 spills at 80 registers; it gets two blocks (119 registers, no spills).
 template<int NT8, bool PRODUCTS> constexpr int bt_min_blocks() { return NT8 == 1 ? 3 : NT8 == 2 ? (PRODUCTS ? 2 : 3) : 1; }
 
-template<int NT8, int RING, bool PRODUCTS>
+template<int NT8, int RING, bool PRODUCTS, bool RAGGED>
 __global__ void __launch_bounds__(BT_NT, bt_min_blocks<NT8, PRODUCTS>())
 k_batched_trial(BatchState S)
 {
   extern __shared__ double sm[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int b = blockIdx.x * BT_WARPS + w;
-  if(b >= S.B || !S.active[b]) return;
-  const int N = S.N, M = S.M;
+  int b = blockIdx.x * BT_WARPS + w;
+  if(b >= S.B) return;
+  if constexpr(RAGGED) b = S.order[b];
+  if(!S.active[b]) return;
+  const int N = S.N, M = RAGGED ? (int)(S.row_off[b + 1] - S.row_off[b]) : S.M;
   constexpr int LD = 8 * NT8 + 1;          // padded row stride of the per-warp matrices
   constexpr int NPAIR = NT8 * (NT8 + 1) / 2;
   double* sA  = sm + (size_t)w * (2 * 8 * NT8 * LD + 6 * BT_NMAX);   // JtJ
@@ -200,8 +211,9 @@ k_batched_trial(BatchState S)
     const int g = lane >> 2, tt = lane & 3;
 
     // ---- one pass over the trial point's Jacobian: JtJ, J'x, |x|^2 ----
-    const double* gJ = S.J + (size_t)b * M * N;
-    const double* gx = S.x + (size_t)b * M;
+    const size_t row0 = RAGGED ? (size_t)S.row_off[b] : (size_t)b * M;
+    const double* gJ = S.J + row0 * N;
+    const double* gx = S.x + row0;
     double acc[NPAIR][2], ag[NT8][2];
 #pragma unroll
     for(int i = 0; i < NPAIR; i++) { acc[i][0] = 0.0; acc[i][1] = 0.0; }
@@ -587,6 +599,12 @@ struct BatchOutlierArgs
   double* scale;              // B, in / out
   double* factors;            // B x nfeat
   int* nfail;
+  // ragged handles (appended, read by the RAGGED instantiations only): problem b's rows are [row_off[b],
+  // row_off[b + 1]) of x, J and factors; nfeat_b: B feature counts (NULL: M_b / fsize); warp slot s takes problem
+  // order[s]
+  const long long* row_off;
+  const int* nfeat_b;
+  const int* order;
 };
 
 // One warp per problem. A_ij of a feature is j_i' inv(JtJ + lambda I) j_j = (L^-1 j_i) . (L^-1 j_j), so one forward
@@ -595,15 +613,26 @@ struct BatchOutlierArgs
 // way (coalesced reads); then lane == measurement substitutes its row against the broadcast L. The next chunk's
 // loads are in flight during the current chunk's substitution. |x|^2 is a fixed-order warp sum and A_01 of a pair
 // takes the neighbouring lane's row by shuffles, so the factors are reproducible bit for bit.
-template<int NT8>
-__global__ void __launch_bounds__(BT_NT) k_batched_outlierness(BatchOutlierArgs A)
+// A ragged problem whose feature count is negative or exceeds its rows gets a NaN scale and no factors. The
+// ragged instantiations ask for one block per SM: left to itself, ptxas gives the NT8 == 3 one 128 registers and
+// 284 bytes of spills (0 with the bound); the uniform ones compile as without a minimum (0).
+template<int NT8, bool RAGGED>
+__global__ void __launch_bounds__(BT_NT, RAGGED ? 1 : 0) k_batched_outlierness(BatchOutlierArgs A)
 {
   extern __shared__ double sm[];
   constexpr int NMAX = 8 * NT8, LD = NMAX + 1;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int b = blockIdx.x * BT_WARPS + w;
+  int b = blockIdx.x * BT_WARPS + w;
   if(b >= A.B) return;
-  const int N = A.N, M = A.M, fs = A.fsize;
+  if constexpr(RAGGED) b = A.order[b];
+  const int N = A.N, M = RAGGED ? (int)(A.row_off[b + 1] - A.row_off[b]) : A.M, fs = A.fsize;
+  const int nfeat = RAGGED ? (A.nfeat_b ? A.nfeat_b[b] : M / fs) : A.nfeat;
+  if constexpr(RAGGED)
+    if(nfeat < 0 || (long long)nfeat * fs > M)
+    {
+      if(lane == 0) A.scale[b] = __longlong_as_double(0x7ff8000000000000LL);
+      return;
+    }
   double* sY  = sm + (size_t)w * (32 * LD + NMAX * LD + NMAX);   // JtJ, then rows of J
   double* sL  = sY + 32 * LD;
   double* srs = sL + NMAX * LD;
@@ -611,8 +640,9 @@ __global__ void __launch_bounds__(BT_NT) k_batched_outlierness(BatchOutlierArgs 
   const bool failed = !isfinite(lam);
   if(lane == 0) { A.lambda[b] = lam; if(failed && A.nfail) atomicAdd(A.nfail, 1); }
 
-  const double* gx = A.x + (size_t)b * M;
-  const double* gJ = A.J + (size_t)b * M * N;
+  const size_t row0 = RAGGED ? (size_t)A.row_off[b] : (size_t)b * M;
+  const double* gx = A.x + row0;
+  const double* gJ = A.J + row0 * N;
   double n2 = 0.0;
   for(int m = lane; m < M; m += 32) { const double v = ldg_stream(gx + m); n2 = fma(v, v, n2); }
   double k = A.scale[b];
@@ -627,8 +657,8 @@ __global__ void __launch_bounds__(BT_NT) k_batched_outlierness(BatchOutlierArgs 
     for(int t = 0; t < NMAX; t++)
       if(t < N && lane + 32 * t < ne) v[t] = ldg_stream(gJ + (size_t)m0 * N + lane + 32 * t);
   };
-  const int Mused = A.nfeat * fs;
-  double* gf = A.factors + (size_t)b * A.nfeat;
+  const int Mused = nfeat * fs;
+  double* gf = A.factors + (RAGGED ? row0 : (size_t)b * A.nfeat);
   load_chunk(0);
   for(int m0 = 0; m0 < Mused; m0 += 32)
   {
@@ -682,19 +712,48 @@ static size_t batched_smem_bytes(int N)
 }
 typedef void (*batched_kernel_t)(BatchState);
 // what the callback hands over; the two products layouts differ in the size of the JtJ buffer
-enum { BF_DENSE = 0, BF_PRODUCTS_FULL = 1, BF_PRODUCTS_PACKED = 2 };
+enum { BF_DENSE = 0, BF_PRODUCTS_FULL = 1, BF_PRODUCTS_PACKED = 2, BF_DENSE_RAGGED = 3 };
+// register-ring variant of the J'J loop (BT_RING row groups in flight; measured in round 2,
+// profiles/r02_variants.txt: 1.37 -> 1.20 ms per trial launch at C3). The products form has no such loop.
+template<int NT8> static batched_kernel_t batched_kernel_nt8(int form)
+{
+  return form == BF_DENSE ? k_batched_trial<NT8, BT_RING, false, false>
+       : form == BF_DENSE_RAGGED ? k_batched_trial<NT8, BT_RING, false, true> : k_batched_trial<NT8, BT_RING, true, false>;
+}
 static batched_kernel_t batched_kernel(int N, int form)
 {
-  // register-ring variant of the J'J loop (BT_RING row groups in flight; measured in round 2,
-  // profiles/r02_variants.txt: 1.37 -> 1.20 ms per trial launch at C3). The products form has no such loop.
-  const bool products = form != BF_DENSE;
   switch((N + 7) / 8)
   {
-  case 1: return products ? k_batched_trial<1, BT_RING, true> : k_batched_trial<1, BT_RING, false>;
-  case 2: return products ? k_batched_trial<2, BT_RING, true> : k_batched_trial<2, BT_RING, false>;
-  case 3: return products ? k_batched_trial<3, BT_RING, true> : k_batched_trial<3, BT_RING, false>;
-  default: return products ? k_batched_trial<4, BT_RING, true> : k_batched_trial<4, BT_RING, false>;
+  case 1: return batched_kernel_nt8<1>(form);
+  case 2: return batched_kernel_nt8<2>(form);
+  case 3: return batched_kernel_nt8<3>(form);
+  default: return batched_kernel_nt8<4>(form);
   }
+}
+
+// The row offsets (B + 1) and the longest-first order (B) of a ragged batch: a stable counting sort of the counts,
+// descending, ties by index, in two passes over 16-bit digits. -1 if a count exceeds INT_MAX.
+extern "C" int dlb_batched_ragged_layout(const unsigned int* Nmeas, unsigned int B, long long* row_off, int* order)
+{
+  row_off[0] = 0;
+  for(unsigned int b = 0; b < B; b++)
+  {
+    if(Nmeas[b] > (unsigned int)INT_MAX) return -1;
+    row_off[b + 1] = row_off[b] + Nmeas[b];
+  }
+  std::vector<int> tmp(B);
+  for(unsigned int b = 0; b < B; b++) order[b] = (int)b;
+  int* src = order; int* dst = tmp.data();
+  for(int shift = 0; shift < 32; shift += 16)
+  {
+    std::vector<unsigned int> pos(65537, 0);
+    auto digit = [&](int b) { return (~Nmeas[b] >> shift) & 0xffffu; };        // ~count: ascending = longest first
+    for(unsigned int i = 0; i < B; i++) pos[digit(src[i]) + 1]++;
+    for(int d = 0; d < 65536; d++) pos[d + 1] += pos[d];
+    for(unsigned int i = 0; i < B; i++) dst[pos[digit(src[i])]++] = src[i];
+    std::swap(src, dst);
+  }
+  return 0;                                                                      // (two passes: src == order)
 }
 
 // Device workspace of the last batched solve, kept for the next one of the same shape and form (the big
@@ -702,6 +761,7 @@ static batched_kernel_t batched_kernel(int N, int form)
 struct BatchWorkspace
 {
   int B = 0, N = 0, M = 0, form = -1, device = -1;
+  long long rows = 0;         // the ragged form's total row count
   std::vector<void*> allocs;
   cudaStream_t st = 0;
   int* h_active = 0;
@@ -712,7 +772,7 @@ struct BatchWorkspace
     allocs.clear();
     if(st) cudaStreamDestroy(st);
     if(h_active) cudaFreeHost(h_active);
-    st = 0; h_active = 0; B = N = M = 0; form = -1; device = -1;
+    st = 0; h_active = 0; B = N = M = 0; rows = 0; form = -1; device = -1;
   }
 };
 static thread_local BatchWorkspace g_ws;
@@ -729,6 +789,12 @@ struct dogleg_gpu_batch
   double* lambda = 0;         // B
   int* status = 0;            // B, DOGLEG_GPU_BATCH_*
   int* nfail = 0;             // 1, for the host-pointer forms
+  // a ragged solve's layout (row_off == NULL: a uniform solve): B + 1 row offsets and the longest-first order on
+  // the device, the counts and their sum on the host
+  long long* row_off = 0;
+  int* order = 0;
+  std::vector<unsigned int> Nmeas;
+  long long rows = 0;
   cudaStream_t st = 0;        // the host-pointer forms run here
   cudaEvent_t ev = 0;         // the handle's last enqueued work: every call is ordered after it
 };
@@ -745,18 +811,20 @@ static void batch_destroy(dogleg_gpu_batch_t* h)
 {
   DeviceScope ds(h->device);
   if(h->ev) cudaEventSynchronize(h->ev);
-  cudaFree(h->JtJ); cudaFree(h->lambda); cudaFree(h->status); cudaFree(h->nfail);
+  cudaFree(h->JtJ); cudaFree(h->lambda); cudaFree(h->status); cudaFree(h->nfail); cudaFree(h->row_off); cudaFree(h->order);
   if(h->st) cudaStreamDestroy(h->st);
   if(h->ev) cudaEventDestroy(h->ev);
   delete h;
 }
 
-static dogleg_gpu_batch_t* batch_create(int device, int B, int N)
+static dogleg_gpu_batch_t* batch_create(int device, int B, int N, bool ragged)
 {
   dogleg_gpu_batch_t* h = new dogleg_gpu_batch_t;
   h->device = device; h->B = B; h->N = N;
   DeviceScope ds(device);
-  if(cudaMalloc((void**)&h->JtJ, (size_t)B * N * N * sizeof(double)) != cudaSuccess ||
+  if((ragged && (cudaMalloc((void**)&h->row_off, ((size_t)B + 1) * sizeof(long long)) != cudaSuccess ||
+                 cudaMalloc((void**)&h->order, (size_t)B * sizeof(int)) != cudaSuccess)) ||
+     cudaMalloc((void**)&h->JtJ, (size_t)B * N * N * sizeof(double)) != cudaSuccess ||
      cudaMalloc((void**)&h->lambda, (size_t)B * sizeof(double)) != cudaSuccess ||
      cudaMalloc((void**)&h->status, (size_t)B * sizeof(int)) != cudaSuccess ||
      cudaMalloc((void**)&h->nfail, sizeof(int)) != cudaSuccess ||
@@ -770,11 +838,16 @@ static dogleg_gpu_batch_t* batch_create(int device, int B, int N)
   return h;
 }
 
-// the solve behind both batched entry points, after their argument checks; M = 0 for the products form
+// the solve behind the batched entry points, after their argument checks; M = 0 for the products and ragged
+// forms. Ragged: Nmeas (B counts) with its host row offsets and order from dlb_batched_ragged_layout.
 static int batched_solve(int form, double* p, int N, int M, unsigned int B, void* f, void* cookie,
                          const dogleg_parameters2_t* parameters, double* norm2x_out, int* iterations_out,
-                         dogleg_gpu_batch_t** returnBatch)
+                         dogleg_gpu_batch_t** returnBatch, const unsigned int* Nmeas = 0,
+                         const long long* h_row_off = 0, const int* h_order = 0)
 {
+  static const char* const name[] = { "dense_batched", "dense_products_batched", "dense_products_batched",
+                                      "dogleg_gpu_optimize_dense_batched_ragged" };
+  const long long rows = form == BF_DENSE_RAGGED ? h_row_off[B] : 0;
   const size_t smem = batched_smem_bytes(N);
   batched_kernel_t kern = batched_kernel(N, form);
   dogleg_parameters2_t P;
@@ -790,7 +863,7 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   BatchWorkspace& W = g_ws;
   int result = -1;
   dogleg_gpu_batch_t* h = 0;
-  if(W.B != (int)B || W.N != N || W.M != M || W.form != form || W.device != dogleg_gpu_get_device())
+  if(W.B != (int)B || W.N != N || W.M != M || W.rows != rows || W.form != form || W.device != dogleg_gpu_get_device())
   {
     W.release();
     W.device = dogleg_gpu_get_device();
@@ -798,6 +871,9 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
     std::vector<size_t> sizes = { bd, bd, bd, bd, bd, bd, bi, bi, bi, bN, bN, bN, bN, bN,
                                   (size_t)B * N * N * sizeof(double), sizeof(int) };
     if(form == BF_DENSE) sizes.insert(sizes.end(), { (size_t)B * M * sizeof(double), (size_t)B * M * N * sizeof(double) });
+    else if(form == BF_DENSE_RAGGED)
+      sizes.insert(sizes.end(), { (size_t)rows * sizeof(double), (size_t)rows * N * sizeof(double),
+                                  ((size_t)B + 1) * sizeof(long long), (size_t)B * sizeof(int) });
     else
     {
       const size_t nS = form == BF_PRODUCTS_PACKED ? (size_t)N * (N + 1) / 2 : (size_t)N * N;
@@ -814,10 +890,10 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
        cudaHostAlloc((void**)&W.h_active, sizeof(int), cudaHostAllocDefault) != cudaSuccess)
     {
       W.release();
-      dlb_set_error(form == BF_DENSE ? "dense_batched: out of device memory" : "dense_products_batched: out of device memory");
+      dlb_set_error((std::string(name[form]) + ": out of device memory").c_str());
       return -1;
     }
-    W.B = (int)B; W.N = N; W.M = M; W.form = form;
+    W.B = (int)B; W.N = N; W.M = M; W.rows = rows; W.form = form;
   }
   {
     void** a = W.allocs.data();
@@ -826,20 +902,23 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
     S.steps = (int*)a[6]; S.flags = (int*)a[7]; S.active = (int*)a[8];
     S.p_before = (double*)a[9]; S.ptrial = (double*)a[10]; S.Jtx = (double*)a[11]; S.cauchy = (double*)a[12];
     S.gn = (double*)a[13]; S.JtJ = (double*)a[14]; S.n_active = (int*)a[15];
-    if(form == BF_DENSE) { S.x = (double*)a[16]; S.J = (double*)a[17]; }
-    else { S.norm2x_in = (double*)a[16]; S.Jtx_in = (double*)a[17]; S.JtJ_in = (double*)a[18]; S.packed = form == BF_PRODUCTS_PACKED; }
+    if(form == BF_DENSE || form == BF_DENSE_RAGGED) { S.x = (double*)a[16]; S.J = (double*)a[17]; }
+    if(form == BF_DENSE_RAGGED) { S.row_off = (const long long*)a[18]; S.order = (const int*)a[19]; }
+    else if(form != BF_DENSE) { S.norm2x_in = (double*)a[16]; S.Jtx_in = (double*)a[17]; S.JtJ_in = (double*)a[18]; S.packed = form == BF_PRODUCTS_PACKED; }
   }
   cudaStream_t st = W.st;
   int* h_active = W.h_active;
   if(returnBatch)
   {
-    h = batch_create(W.device, (int)B, N);
+    h = batch_create(W.device, (int)B, N, form == BF_DENSE_RAGGED);
     if(!h)
     {
       dlb_set_error(form == BF_DENSE ? "dense_batched2: out of device memory for the returned batch"
-                                     : "dense_products_batched2: out of device memory for the returned batch");
+                    : form == BF_DENSE_RAGGED ? "dogleg_gpu_optimize_dense_batched_ragged: out of device memory for the returned batch"
+                                              : "dense_products_batched2: out of device memory for the returned batch");
       return -1;
     }
+    if(form == BF_DENSE_RAGGED) { h->Nmeas.assign(Nmeas, Nmeas + B); h->rows = rows; }
     S.status = h->status;
     CUB(cudaMemsetAsync(S.status, 0, (size_t)B * sizeof(int), st));
   }
@@ -849,6 +928,11 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   CUB(cudaMemsetAsync(S.lambda, 0, (size_t)B * sizeof(double), st));
   CUB(cudaMemsetAsync(S.steps, 0, (size_t)B * sizeof(int), st));
   CUB(cudaMemsetAsync(S.flags, 0, (size_t)B * sizeof(int), st));
+  if(form == BF_DENSE_RAGGED)
+  {
+    CUB(cudaMemcpyAsync((void*)S.row_off, h_row_off, ((size_t)B + 1) * sizeof(long long), cudaMemcpyHostToDevice, st));
+    CUB(cudaMemcpyAsync((void*)S.order, h_order, (size_t)B * sizeof(int), cudaMemcpyHostToDevice, st));
+  }
   {
     std::vector<double> tr(B, S.tr0);
     std::vector<int> ones(B, 1);
@@ -872,6 +956,8 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
       cudaEventRecord(ev[0], st);
       if(form == BF_DENSE)
         ((dogleg_gpu_callback_dense_batched_t*)f)(S.ptrial, S.x, S.J, S.active, (int)B, (void*)st, cookie);
+      else if(form == BF_DENSE_RAGGED)
+        ((dogleg_gpu_callback_dense_ragged_t*)f)(S.ptrial, S.x, S.J, S.row_off, S.active, (int)B, (void*)st, cookie);
       else
         ((dogleg_gpu_callback_dense_products_batched_t*)f)(S.ptrial, S.norm2x_in, S.Jtx_in, S.JtJ_in, S.active, (int)B,
                                                             (void*)st, cookie);
@@ -894,6 +980,11 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   {
     CUB(cudaMemcpyAsync(h->JtJ, S.JtJ, (size_t)B * N * N * sizeof(double), cudaMemcpyDeviceToDevice, st));
     CUB(cudaMemcpyAsync(h->lambda, S.lambda, (size_t)B * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    if(form == BF_DENSE_RAGGED)
+    {
+      CUB(cudaMemcpyAsync(h->row_off, S.row_off, ((size_t)B + 1) * sizeof(long long), cudaMemcpyDeviceToDevice, st));
+      CUB(cudaMemcpyAsync(h->order, S.order, (size_t)B * sizeof(int), cudaMemcpyDeviceToDevice, st));
+    }
   }
   CUB(cudaStreamSynchronize(st));
   result = (int)B - *h_active;
@@ -999,6 +1090,7 @@ static bool outlier_args_ok(const char* fn, const dogleg_gpu_batch_t* h, const v
   std::string msg;
   if(featureSize <= 1) featureSize = 1;
   if(!h) msg = "NULL handle";
+  else if(h->row_off) msg = "the handle is from a ragged solve: use dogleg_gpu_batch_outlierness_ragged";
   else if(!x || !J || !scale || !factors) msg = "bad arguments (needs x, J, scale and factors)";
   else if(featureSize > 2) msg = "featureSize > 2 not implemented yet. Got featureSize=" + std::to_string(featureSize);
   else if(Nfeatures < 1 || Nmeas < 1 || Nmeas > (unsigned int)INT_MAX) msg = "bad arguments (needs Nfeatures >= 1 and Nmeas >= 1)";
@@ -1009,16 +1101,22 @@ static bool outlier_args_ok(const char* fn, const dogleg_gpu_batch_t* h, const v
 }
 
 // enqueue k_batched_outlierness on st, after the handle's earlier work; it becomes the handle's latest
-static int batch_outlier_enqueue(dogleg_gpu_batch_t* h, const double* d_x, const double* d_J, int M, int fsize,
-                                 int nfeat, const int* d_nout, double* d_scale, double* d_factors, int* nfail,
-                                 cudaStream_t st)
+// (a ragged handle: M and nfeat unused, d_nfeat its B feature counts or NULL)
+typedef void (*outlier_kernel_t)(BatchOutlierArgs);
+template<bool RAGGED> static outlier_kernel_t outlier_kernel(int nt8)
 {
-  typedef void (*outlier_kernel_t)(BatchOutlierArgs);
+  return nt8 == 1 ? k_batched_outlierness<1, RAGGED> : nt8 == 2 ? k_batched_outlierness<2, RAGGED>
+       : nt8 == 3 ? k_batched_outlierness<3, RAGGED> : k_batched_outlierness<4, RAGGED>;
+}
+static int batch_outlier_enqueue(dogleg_gpu_batch_t* h, const double* d_x, const double* d_J, int M, int fsize,
+                                 int nfeat, const int* d_nfeat, const int* d_nout, double* d_scale, double* d_factors,
+                                 int* nfail, cudaStream_t st)
+{
   const int nt8 = (h->N + 7) / 8, ld = 8 * nt8 + 1;
-  const outlier_kernel_t kern = nt8 == 1 ? k_batched_outlierness<1> : nt8 == 2 ? k_batched_outlierness<2>
-                              : nt8 == 3 ? k_batched_outlierness<3> : k_batched_outlierness<4>;
+  const outlier_kernel_t kern = h->row_off ? outlier_kernel<true>(nt8) : outlier_kernel<false>(nt8);
   const size_t smem = sizeof(double) * (size_t)BT_WARPS * (32 * ld + 8 * nt8 * ld + 8 * nt8);
-  BatchOutlierArgs A = { h->B, h->N, M, fsize, nfeat, h->JtJ, h->lambda, d_x, d_J, d_nout, d_scale, d_factors, nfail };
+  BatchOutlierArgs A = { h->B, h->N, M, fsize, nfeat, h->JtJ, h->lambda, d_x, d_J, d_nout, d_scale, d_factors, nfail,
+                         h->row_off, d_nfeat, h->order };
   CUB(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   CUB(cudaStreamWaitEvent(st, h->ev, 0));
   kern<<<(h->B + BT_WARPS - 1) / BT_WARPS, BT_NT, smem, st>>>(A);
@@ -1053,7 +1151,7 @@ extern "C" int dogleg_gpu_batch_outlierness(dogleg_gpu_batch_t* h, const double*
   }
   CUB(cudaStreamWaitEvent(h->st, h->ev, 0));
   CUB(cudaMemsetAsync(h->nfail, 0, sizeof(int), h->st));
-  if(batch_outlier_enqueue(h, dx, dJ, (int)Nmeas, featureSize, Nfeatures, dnout, dscale, df, h->nfail, h->st)) goto fail;
+  if(batch_outlier_enqueue(h, dx, dJ, (int)Nmeas, featureSize, Nfeatures, 0, dnout, dscale, df, h->nfail, h->st)) goto fail;
   CUB(cudaMemcpyAsync(factors, df, nf * sizeof(double), cudaMemcpyDeviceToHost, h->st));
   CUB(cudaMemcpyAsync(scale, dscale, B * sizeof(double), cudaMemcpyDeviceToHost, h->st));
   CUB(cudaMemcpyAsync(&nfail, h->nfail, sizeof(int), cudaMemcpyDeviceToHost, h->st));
@@ -1073,8 +1171,86 @@ extern "C" int dogleg_gpu_batch_outlierness_device(dogleg_gpu_batch_t* h, const 
                       Nfeatures))
     return -1;
   DeviceScope ds(h->device);
-  return batch_outlier_enqueue(h, d_x, d_J, (int)Nmeas, featureSize, Nfeatures, d_NoutlierFeatures, d_scale, d_factors,
-                               0, (cudaStream_t)stream);
+  return batch_outlier_enqueue(h, d_x, d_J, (int)Nmeas, featureSize, Nfeatures, 0, d_NoutlierFeatures, d_scale,
+                               d_factors, 0, (cudaStream_t)stream);
+}
+
+// the argument checks of both ragged outlierness calls; featureSize <= 1 means 1
+static bool outlier_ragged_args_ok(const char* fn, const dogleg_gpu_batch_t* h, const void* x, const void* J,
+                                   const void* scale, const void* factors, int& featureSize)
+{
+  std::string msg;
+  if(featureSize <= 1) featureSize = 1;
+  if(!h) msg = "NULL handle";
+  else if(!h->row_off) msg = "the handle is from a uniform batched solve: use dogleg_gpu_batch_outlierness";
+  else if(!x || !J || !scale || !factors) msg = "bad arguments (needs x, J, scale and factors)";
+  else if(featureSize > 2) msg = "featureSize > 2 not implemented yet. Got featureSize=" + std::to_string(featureSize);
+  if(msg.empty()) return true;
+  dlb_set_error((std::string(fn) + ": " + msg).c_str());
+  return false;
+}
+
+extern "C" int dogleg_gpu_batch_outlierness_ragged(dogleg_gpu_batch_t* h, const double* x, const double* J,
+                                                   int featureSize, const int* Nfeatures, const int* NoutlierFeatures,
+                                                   double* scale, double* factors)
+{
+  static const char* fn = "dogleg_gpu_batch_outlierness_ragged";
+  if(!outlier_ragged_args_ok(fn, h, x, J, scale, factors, featureSize)) return -1;
+  if(Nfeatures)
+    for(int b = 0; b < h->B; b++)
+      if(Nfeatures[b] < 0 || (long long)Nfeatures[b] * featureSize > (long long)h->Nmeas[b])
+      {
+        dlb_set_error((std::string(fn) + ": Nfeatures[b]*featureSize must be in 0..Nmeas[b]; b = " + std::to_string(b) +
+                       ", Nfeatures[b] = " + std::to_string(Nfeatures[b]) + ", Nmeas[b] = " +
+                       std::to_string(h->Nmeas[b])).c_str());
+        return -1;
+      }
+  DeviceScope ds(h->device);
+  const size_t B = (size_t)h->B, nx = (size_t)h->rows, nJ = nx * h->N;
+  double *dx = 0, *dJ = 0, *dscale = 0, *df = 0;
+  int *dnfeat = 0, *dnout = 0;
+  int nfail = 0, result = -1;
+  CUB(cudaMalloc((void**)&dx, (nx ? nx : 1) * sizeof(double)));
+  CUB(cudaMalloc((void**)&dJ, (nJ ? nJ : 1) * sizeof(double)));
+  CUB(cudaMalloc((void**)&dscale, B * sizeof(double)));
+  CUB(cudaMalloc((void**)&df, (nx ? nx : 1) * sizeof(double)));
+  CUB(cudaMemcpyAsync(dx, x, nx * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  CUB(cudaMemcpyAsync(dJ, J, nJ * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  CUB(cudaMemcpyAsync(dscale, scale, B * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  CUB(cudaMemcpyAsync(df, factors, nx * sizeof(double), cudaMemcpyHostToDevice, h->st));     // rows that are no feature stay
+  if(Nfeatures)
+  {
+    CUB(cudaMalloc((void**)&dnfeat, B * sizeof(int)));
+    CUB(cudaMemcpyAsync(dnfeat, Nfeatures, B * sizeof(int), cudaMemcpyHostToDevice, h->st));
+  }
+  if(NoutlierFeatures)
+  {
+    CUB(cudaMalloc((void**)&dnout, B * sizeof(int)));
+    CUB(cudaMemcpyAsync(dnout, NoutlierFeatures, B * sizeof(int), cudaMemcpyHostToDevice, h->st));
+  }
+  CUB(cudaStreamWaitEvent(h->st, h->ev, 0));
+  CUB(cudaMemsetAsync(h->nfail, 0, sizeof(int), h->st));
+  if(batch_outlier_enqueue(h, dx, dJ, 0, featureSize, 0, dnfeat, dnout, dscale, df, h->nfail, h->st)) goto fail;
+  CUB(cudaMemcpyAsync(factors, df, nx * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaMemcpyAsync(scale, dscale, B * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaMemcpyAsync(&nfail, h->nfail, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+  CUB(cudaStreamSynchronize(h->st));
+  result = nfail;
+fail:
+  cudaFree(dx); cudaFree(dJ); cudaFree(dscale); cudaFree(df); cudaFree(dnfeat); cudaFree(dnout);
+  return result;
+}
+
+extern "C" int dogleg_gpu_batch_outlierness_ragged_device(dogleg_gpu_batch_t* h, const double* d_x, const double* d_J,
+                                                          int featureSize, const int* d_Nfeatures,
+                                                          const int* d_NoutlierFeatures, double* d_scale,
+                                                          double* d_factors, void* stream)
+{
+  if(!outlier_ragged_args_ok("dogleg_gpu_batch_outlierness_ragged_device", h, d_x, d_J, d_scale, d_factors, featureSize))
+    return -1;
+  DeviceScope ds(h->device);
+  return batch_outlier_enqueue(h, d_x, d_J, 0, featureSize, 0, d_Nfeatures, d_NoutlierFeatures, d_scale, d_factors, 0,
+                               (cudaStream_t)stream);
 }
 
 extern "C" void dogleg_gpu_batch_free(dogleg_gpu_batch_t** batch)
@@ -1109,6 +1285,40 @@ extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate,
                                                  double* norm2x_out, int* iterations_out)
 {
   return dogleg_gpu_optimize_dense_batched2(p, Nstate, Nmeas, B, f, cookie, parameters, norm2x_out, iterations_out, 0);
+}
+
+extern "C" int dogleg_gpu_optimize_dense_batched_ragged(double* p, unsigned int Nstate, const unsigned int* Nmeas,
+                                                        unsigned int B, dogleg_gpu_callback_dense_ragged_t* f,
+                                                        void* cookie, const dogleg_parameters2_t* parameters,
+                                                        double* norm2x_out, int* iterations_out,
+                                                        dogleg_gpu_batch_t** returnBatch)
+{
+  static const std::string fn = "dogleg_gpu_optimize_dense_batched_ragged: ";
+  if(returnBatch) *returnBatch = 0;
+  if(dogleg_gpu_device_count() <= 0) { dlb_set_error((fn + "no CUDA device available: libdogleg-b200 has no CPU fallback").c_str()); return -1; }
+  if(!f || !p || !Nmeas || B == 0) { dlb_set_error((fn + "bad arguments (needs p, Nmeas, a callback and B > 0)").c_str()); return -1; }
+  const int N = (int)Nstate;
+  if(N > BT_NMAX || N < 1)
+  {
+    dlb_set_error((fn + "needs 1 <= Nstate <= 32; use dogleg_optimize_dense2 per problem for bigger ones").c_str());
+    return -1;
+  }
+  std::vector<long long> row_off((size_t)B + 1);
+  std::vector<int> order(B);
+  if(dlb_batched_ragged_layout(Nmeas, B, row_off.data(), order.data()) != 0)
+  {
+    unsigned int b = 0;
+    while(Nmeas[b] <= (unsigned int)INT_MAX) b++;
+    dlb_set_error((fn + "Nmeas[" + std::to_string(b) + "] = " + std::to_string(Nmeas[b]) + " exceeds INT_MAX").c_str());
+    return -1;
+  }
+  if(row_off[B] > (long long)(SIZE_MAX / sizeof(double) / (N + 1)))
+  {
+    dlb_set_error((fn + "out of device memory").c_str());
+    return -1;
+  }
+  return batched_solve(BF_DENSE_RAGGED, p, N, 0, B, (void*)f, cookie, parameters, norm2x_out, iterations_out,
+                       returnBatch, Nmeas, row_off.data(), order.data());
 }
 
 extern "C" int dogleg_gpu_optimize_dense_products_batched2(double* p, unsigned int Nstate, unsigned int B,

@@ -136,6 +136,15 @@ def load():
     L.dogleg_gpu_batch_outlierness.restype = C.c_int
     L.dogleg_gpu_batch_outlierness_device.argtypes = [vp, vp, vp, C.c_uint, C.c_int, C.c_int, vp, vp, vp, vp]
     L.dogleg_gpu_batch_outlierness_device.restype = C.c_int
+    L.dogleg_gpu_optimize_dense_batched_ragged.argtypes = [dp, C.c_uint, C.POINTER(C.c_uint), C.c_uint, vp, vp, PP, dp, ip,
+                                                           C.POINTER(vp)]
+    L.dogleg_gpu_optimize_dense_batched_ragged.restype = C.c_int
+    L.dlb_batched_ragged_layout.argtypes = [C.POINTER(C.c_uint), C.c_uint, C.POINTER(C.c_longlong), ip]
+    L.dlb_batched_ragged_layout.restype = C.c_int
+    L.dogleg_gpu_batch_outlierness_ragged.argtypes = [vp, dp, dp, C.c_int, ip, ip, dp, dp]
+    L.dogleg_gpu_batch_outlierness_ragged.restype = C.c_int
+    L.dogleg_gpu_batch_outlierness_ragged_device.argtypes = [vp, vp, vp, C.c_int, vp, vp, vp, vp, vp]
+    L.dogleg_gpu_batch_outlierness_ragged_device.restype = C.c_int
     L.dogleg_gpu_batch_free.argtypes = [C.POINTER(vp)]
     L.dogleg_gpu_batch_free.restype = None
     L.dogleg_gpu_release_batched_cache.restype = None
