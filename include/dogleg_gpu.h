@@ -213,6 +213,31 @@ int dogleg_gpu_optimize_dense_batched_ragged(double* p, unsigned int Nstate, con
  * first, ties by index (the order in which the trial kernel's warps take them). -1 if a count exceeds INT_MAX. */
 int dlb_batched_ragged_layout(const unsigned int* Nmeas, unsigned int B, long long* row_off, int* order);
 
+/* Batched dense solves with a single-precision Jacobian: dogleg_gpu_optimize_dense_batched2 and
+ * dogleg_gpu_optimize_dense_batched_ragged with d_J in float, in the same layout. Everything else -- p, x, |x|^2,
+ * every internal quantity and everything a returned handle holds -- stays double, and the parameters, return value,
+ * d_active, the handle and the refusals are those of the double entry points (error messages name these functions).
+ * The solver widens each float to double (exact) and then runs the double kernel's operations in the same order, so
+ * the results are those of the double entry point on the same batch with J widened to double, bit for bit, and a
+ * handle from a float solve is indistinguishable from one from that double solve (outlierness calls take the widened
+ * J). The gradient test and the step are formed from the float Jacobian the callback supplied: the solver converges
+ * to that model's fixed point J_f'x = 0, not to the fixed point of an unrounded Jacobian it never sees. The callback
+ * writes 4 bytes per entry of J instead of 8, and the solver streams half the Jacobian bytes. */
+typedef void (dogleg_gpu_callback_dense_batched_f32jac_t)(const double* d_p, double* d_x, float* d_J,
+                                                          const int* d_active, int B, void* stream, void* cookie);
+int dogleg_gpu_optimize_dense_batched_f32jac(double* p, unsigned int Nstate, unsigned int Nmeas, unsigned int B,
+                                             dogleg_gpu_callback_dense_batched_f32jac_t* f, void* cookie,
+                                             const dogleg_parameters2_t* parameters, double* norm2x_out,
+                                             int* iterations_out, dogleg_gpu_batch_t** returnBatch);
+typedef void (dogleg_gpu_callback_dense_ragged_f32jac_t)(const double* d_p, double* d_x, float* d_J,
+                                                         const long long* d_row_off, const int* d_active, int B,
+                                                         void* stream, void* cookie);
+int dogleg_gpu_optimize_dense_batched_ragged_f32jac(double* p, unsigned int Nstate, const unsigned int* Nmeas,
+                                                    unsigned int B, dogleg_gpu_callback_dense_ragged_f32jac_t* f,
+                                                    void* cookie, const dogleg_parameters2_t* parameters,
+                                                    double* norm2x_out, int* iterations_out,
+                                                    dogleg_gpu_batch_t** returnBatch);
+
 /* Why a problem stopped, in the order the single-problem solver tests (dogleg_core.c run_solver): after an
  * accepted step the gradient test comes before the iteration cap; at the initial point a problem is
  * GRADIENT if it has converged, else MAX_ITERATIONS if max_iterations <= 0. */

@@ -33,6 +33,10 @@
 // Ragged form (dogleg_gpu_optimize_dense_batched_ragged): problem b has its own number of measurements, its rows
 // at row_off[b] of x and J. The RAGGED instantiations of the same two kernels take each warp's M and row pointers
 // from the offsets and its problem from a longest-first order; everything else is the uniform code.
+//
+// Float-Jacobian forms (dogleg_gpu_optimize_dense_batched_f32jac, _ragged_f32jac): the callback writes J in float,
+// which halves the bytes of the stream. The float instantiations load it as float and widen every value to double
+// before it is used, so they compute exactly what the double kernel computes on the widened J.
 #include "dlb_common.cuh"
 #include "dogleg_gpu.h"
 #include "dlb_outlier_math.h"
@@ -42,6 +46,7 @@
 #include <algorithm>
 #include <climits>
 #include <cstdint>
+#include <type_traits>
 
 extern "C" void dlb_set_error(const char* msg);
 
@@ -74,6 +79,8 @@ struct BatchState
   // [row_off[b], row_off[b + 1]) of x and J; warp slot s takes problem order[s], longest first
   const long long *row_off;
   const int *order;
+  // the f32jac forms' Jacobian (appended likewise, read by the float instantiations only): J in float, in J's layout
+  float *Jf;
 };
 enum { FL_CAUCHY = 1, FL_GN = 2, FL_EDGE = 4, FL_PENDING = 8 };
 
@@ -160,7 +167,10 @@ __device__ __forceinline__ void bt_cholesky_ladder(const double* sA, double* sL,
 // products form at NT8 == 2 spills at 80 registers; it gets two blocks (119 registers, no spills).
 template<int NT8, bool PRODUCTS> constexpr int bt_min_blocks() { return NT8 == 1 ? 3 : NT8 == 2 ? (PRODUCTS ? 2 : 3) : 1; }
 
-template<int NT8, int RING, bool PRODUCTS, bool RAGGED>
+// JT: the element type of the callback's Jacobian (double, or float for the f32jac forms). Only the loads see it:
+// every value is widened to double before it enters a DMMA or an FMA, and the sums run in the same order, so a
+// float J gives the results of the double kernel on the widened J, bit for bit.
+template<int NT8, int RING, bool PRODUCTS, bool RAGGED, typename JT = double>
 __global__ void __launch_bounds__(BT_NT, bt_min_blocks<NT8, PRODUCTS>())
 k_batched_trial(BatchState S)
 {
@@ -212,7 +222,8 @@ k_batched_trial(BatchState S)
 
     // ---- one pass over the trial point's Jacobian: JtJ, J'x, |x|^2 ----
     const size_t row0 = RAGGED ? (size_t)S.row_off[b] : (size_t)b * M;
-    const double* gJ = S.J + row0 * N;
+    const JT* gJ;
+    if constexpr(std::is_same<JT, float>::value) gJ = S.Jf + row0 * N; else gJ = S.J + row0 * N;
     const double* gx = S.x + row0;
     double acc[NPAIR][2], ag[NT8][2];
 #pragma unroll
@@ -221,12 +232,12 @@ k_batched_trial(BatchState S)
     for(int i = 0; i < NT8; i++) { ag[i][0] = 0.0; ag[i][1] = 0.0; }
     double n2 = 0.0;
     // one 4-row group: this lane's entries of the group's rows (zeros beyond the last row)
-    auto load_group = [&](int r0, double (&v)[NT8], double& xr) {
+    auto load_group = [&](int r0, JT (&v)[NT8], double& xr) {
       const int row = r0 + tt;
       const bool valid = row < M;
       xr = valid ? ldg_stream(gx + row) : 0.0;
 #pragma unroll
-      for(int ti = 0; ti < NT8; ti++) v[ti] = (valid && 8 * ti + g < N) ? ldg_stream(gJ + (size_t)row * N + 8 * ti + g) : 0.0;
+      for(int ti = 0; ti < NT8; ti++) v[ti] = (valid && 8 * ti + g < N) ? ldg_stream(gJ + (size_t)row * N + 8 * ti + g) : JT(0);
     };
     auto use_group = [&](const double (&v)[NT8], double xr) {
       // J'x by plain multiply-adds (this lane's row of the group times its x; the four lanes of a state are
@@ -249,8 +260,10 @@ k_batched_trial(BatchState S)
     if(RING > 1)
     { // register ring: the loads of group i + RING are issued before the DMMAs of group i, so RING
       // groups (3 * RING loads per lane) are in flight; groups are consumed in the same order as
-      // below, hence bit-identical sums. Groups past the end are zeros.
-      double vb[RING > 1 ? RING : 1][NT8], xb[RING > 1 ? RING : 1];
+      // below, hence bit-identical sums. Groups past the end are zeros. The ring holds J as loaded (a float ring
+      // takes half the registers) and widens on use.
+      JT vb[RING > 1 ? RING : 1][NT8];
+      double xb[RING > 1 ? RING : 1];
 #pragma unroll
       for(int u = 0; u < RING; u++) load_group(4 * u, vb[u], xb[u]);
       for(int r0 = 0; r0 < M; r0 += 4 * RING)
@@ -272,8 +285,11 @@ k_batched_trial(BatchState S)
 #pragma unroll 8
       for(int r0 = 0; r0 < M; r0 += 4)
       {
+        JT vj[NT8];
         double v[NT8], xr;
-        load_group(r0, v, xr);
+        load_group(r0, vj, xr);
+#pragma unroll
+        for(int ti = 0; ti < NT8; ti++) v[ti] = vj[ti];
         use_group(v, xr);
       }
     }
@@ -712,13 +728,22 @@ static size_t batched_smem_bytes(int N)
 }
 typedef void (*batched_kernel_t)(BatchState);
 // what the callback hands over; the two products layouts differ in the size of the JtJ buffer
-enum { BF_DENSE = 0, BF_PRODUCTS_FULL = 1, BF_PRODUCTS_PACKED = 2, BF_DENSE_RAGGED = 3 };
+enum { BF_DENSE = 0, BF_PRODUCTS_FULL = 1, BF_PRODUCTS_PACKED = 2, BF_DENSE_RAGGED = 3, BF_DENSE_F32 = 4,
+       BF_DENSE_RAGGED_F32 = 5 };
+static bool bf_ragged(int form) { return form == BF_DENSE_RAGGED || form == BF_DENSE_RAGGED_F32; }
+static bool bf_f32(int form) { return form == BF_DENSE_F32 || form == BF_DENSE_RAGGED_F32; }
 // register-ring variant of the J'J loop (BT_RING row groups in flight; measured in round 2,
 // profiles/r02_variants.txt: 1.37 -> 1.20 ms per trial launch at C3). The products form has no such loop.
 template<int NT8> static batched_kernel_t batched_kernel_nt8(int form)
 {
-  return form == BF_DENSE ? k_batched_trial<NT8, BT_RING, false, false>
-       : form == BF_DENSE_RAGGED ? k_batched_trial<NT8, BT_RING, false, true> : k_batched_trial<NT8, BT_RING, true, false>;
+  switch(form)
+  {
+  case BF_DENSE: return k_batched_trial<NT8, BT_RING, false, false>;
+  case BF_DENSE_RAGGED: return k_batched_trial<NT8, BT_RING, false, true>;
+  case BF_DENSE_F32: return k_batched_trial<NT8, BT_RING, false, false, float>;
+  case BF_DENSE_RAGGED_F32: return k_batched_trial<NT8, BT_RING, false, true, float>;
+  default: return k_batched_trial<NT8, BT_RING, true, false>;
+  }
 }
 static batched_kernel_t batched_kernel(int N, int form)
 {
@@ -846,8 +871,11 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
                          const long long* h_row_off = 0, const int* h_order = 0)
 {
   static const char* const name[] = { "dense_batched", "dense_products_batched", "dense_products_batched",
-                                      "dogleg_gpu_optimize_dense_batched_ragged" };
-  const long long rows = form == BF_DENSE_RAGGED ? h_row_off[B] : 0;
+                                      "dogleg_gpu_optimize_dense_batched_ragged",
+                                      "dogleg_gpu_optimize_dense_batched_f32jac",
+                                      "dogleg_gpu_optimize_dense_batched_ragged_f32jac" };
+  const bool ragged = bf_ragged(form), f32 = bf_f32(form);
+  const long long rows = ragged ? h_row_off[B] : 0;
   const size_t smem = batched_smem_bytes(N);
   batched_kernel_t kern = batched_kernel(N, form);
   dogleg_parameters2_t P;
@@ -870,9 +898,10 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
     const size_t bN = (size_t)B * N * sizeof(double), bd = (size_t)B * sizeof(double), bi = (size_t)B * sizeof(int);
     std::vector<size_t> sizes = { bd, bd, bd, bd, bd, bd, bi, bi, bi, bN, bN, bN, bN, bN,
                                   (size_t)B * N * N * sizeof(double), sizeof(int) };
-    if(form == BF_DENSE) sizes.insert(sizes.end(), { (size_t)B * M * sizeof(double), (size_t)B * M * N * sizeof(double) });
-    else if(form == BF_DENSE_RAGGED)
-      sizes.insert(sizes.end(), { (size_t)rows * sizeof(double), (size_t)rows * N * sizeof(double),
+    const size_t jsz = f32 ? sizeof(float) : sizeof(double);          // an entry of J
+    if(form == BF_DENSE || form == BF_DENSE_F32) sizes.insert(sizes.end(), { (size_t)B * M * sizeof(double), (size_t)B * M * N * jsz });
+    else if(ragged)
+      sizes.insert(sizes.end(), { (size_t)rows * sizeof(double), (size_t)rows * N * jsz,
                                   ((size_t)B + 1) * sizeof(long long), (size_t)B * sizeof(int) });
     else
     {
@@ -902,23 +931,26 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
     S.steps = (int*)a[6]; S.flags = (int*)a[7]; S.active = (int*)a[8];
     S.p_before = (double*)a[9]; S.ptrial = (double*)a[10]; S.Jtx = (double*)a[11]; S.cauchy = (double*)a[12];
     S.gn = (double*)a[13]; S.JtJ = (double*)a[14]; S.n_active = (int*)a[15];
-    if(form == BF_DENSE || form == BF_DENSE_RAGGED) { S.x = (double*)a[16]; S.J = (double*)a[17]; }
-    if(form == BF_DENSE_RAGGED) { S.row_off = (const long long*)a[18]; S.order = (const int*)a[19]; }
-    else if(form != BF_DENSE) { S.norm2x_in = (double*)a[16]; S.Jtx_in = (double*)a[17]; S.JtJ_in = (double*)a[18]; S.packed = form == BF_PRODUCTS_PACKED; }
+    if(form == BF_DENSE || ragged || f32)
+    {
+      S.x = (double*)a[16];
+      if(f32) S.Jf = (float*)a[17]; else S.J = (double*)a[17];
+    }
+    if(ragged) { S.row_off = (const long long*)a[18]; S.order = (const int*)a[19]; }
+    else if(form != BF_DENSE && form != BF_DENSE_F32) { S.norm2x_in = (double*)a[16]; S.Jtx_in = (double*)a[17]; S.JtJ_in = (double*)a[18]; S.packed = form == BF_PRODUCTS_PACKED; }
   }
   cudaStream_t st = W.st;
   int* h_active = W.h_active;
   if(returnBatch)
   {
-    h = batch_create(W.device, (int)B, N, form == BF_DENSE_RAGGED);
+    h = batch_create(W.device, (int)B, N, ragged);
     if(!h)
     {
-      dlb_set_error(form == BF_DENSE ? "dense_batched2: out of device memory for the returned batch"
-                    : form == BF_DENSE_RAGGED ? "dogleg_gpu_optimize_dense_batched_ragged: out of device memory for the returned batch"
-                                              : "dense_products_batched2: out of device memory for the returned batch");
+      const std::string who = form == BF_DENSE ? "dense_batched2" : ragged || f32 ? name[form] : "dense_products_batched2";
+      dlb_set_error((who + ": out of device memory for the returned batch").c_str());
       return -1;
     }
-    if(form == BF_DENSE_RAGGED) { h->Nmeas.assign(Nmeas, Nmeas + B); h->rows = rows; }
+    if(ragged) { h->Nmeas.assign(Nmeas, Nmeas + B); h->rows = rows; }
     S.status = h->status;
     CUB(cudaMemsetAsync(S.status, 0, (size_t)B * sizeof(int), st));
   }
@@ -928,7 +960,7 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   CUB(cudaMemsetAsync(S.lambda, 0, (size_t)B * sizeof(double), st));
   CUB(cudaMemsetAsync(S.steps, 0, (size_t)B * sizeof(int), st));
   CUB(cudaMemsetAsync(S.flags, 0, (size_t)B * sizeof(int), st));
-  if(form == BF_DENSE_RAGGED)
+  if(ragged)
   {
     CUB(cudaMemcpyAsync((void*)S.row_off, h_row_off, ((size_t)B + 1) * sizeof(long long), cudaMemcpyHostToDevice, st));
     CUB(cudaMemcpyAsync((void*)S.order, h_order, (size_t)B * sizeof(int), cudaMemcpyHostToDevice, st));
@@ -958,6 +990,11 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
         ((dogleg_gpu_callback_dense_batched_t*)f)(S.ptrial, S.x, S.J, S.active, (int)B, (void*)st, cookie);
       else if(form == BF_DENSE_RAGGED)
         ((dogleg_gpu_callback_dense_ragged_t*)f)(S.ptrial, S.x, S.J, S.row_off, S.active, (int)B, (void*)st, cookie);
+      else if(form == BF_DENSE_F32)
+        ((dogleg_gpu_callback_dense_batched_f32jac_t*)f)(S.ptrial, S.x, S.Jf, S.active, (int)B, (void*)st, cookie);
+      else if(form == BF_DENSE_RAGGED_F32)
+        ((dogleg_gpu_callback_dense_ragged_f32jac_t*)f)(S.ptrial, S.x, S.Jf, S.row_off, S.active, (int)B, (void*)st,
+                                                         cookie);
       else
         ((dogleg_gpu_callback_dense_products_batched_t*)f)(S.ptrial, S.norm2x_in, S.Jtx_in, S.JtJ_in, S.active, (int)B,
                                                             (void*)st, cookie);
@@ -980,7 +1017,7 @@ static int batched_solve(int form, double* p, int N, int M, unsigned int B, void
   {
     CUB(cudaMemcpyAsync(h->JtJ, S.JtJ, (size_t)B * N * N * sizeof(double), cudaMemcpyDeviceToDevice, st));
     CUB(cudaMemcpyAsync(h->lambda, S.lambda, (size_t)B * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    if(form == BF_DENSE_RAGGED)
+    if(ragged)
     {
       CUB(cudaMemcpyAsync(h->row_off, S.row_off, ((size_t)B + 1) * sizeof(long long), cudaMemcpyDeviceToDevice, st));
       CUB(cudaMemcpyAsync(h->order, S.order, (size_t)B * sizeof(int), cudaMemcpyDeviceToDevice, st));
@@ -1287,13 +1324,14 @@ extern "C" int dogleg_gpu_optimize_dense_batched(double* p, unsigned int Nstate,
   return dogleg_gpu_optimize_dense_batched2(p, Nstate, Nmeas, B, f, cookie, parameters, norm2x_out, iterations_out, 0);
 }
 
-extern "C" int dogleg_gpu_optimize_dense_batched_ragged(double* p, unsigned int Nstate, const unsigned int* Nmeas,
-                                                        unsigned int B, dogleg_gpu_callback_dense_ragged_t* f,
-                                                        void* cookie, const dogleg_parameters2_t* parameters,
-                                                        double* norm2x_out, int* iterations_out,
-                                                        dogleg_gpu_batch_t** returnBatch)
+// The checks and the host layout of both ragged entry points (form: BF_DENSE_RAGGED or BF_DENSE_RAGGED_F32), then the
+// solve. Refuses, before the first callback and naming the entry point: Nstate outside 1..32, B == 0, a NULL p, Nmeas
+// or callback, a count above INT_MAX and a batch whose x and J would not fit in a size_t.
+static int ragged_solve(int form, const char* entry, double* p, unsigned int Nstate, const unsigned int* Nmeas,
+                        unsigned int B, void* f, void* cookie, const dogleg_parameters2_t* parameters, double* norm2x_out,
+                        int* iterations_out, dogleg_gpu_batch_t** returnBatch)
 {
-  static const std::string fn = "dogleg_gpu_optimize_dense_batched_ragged: ";
+  const std::string fn = std::string(entry) + ": ";
   if(returnBatch) *returnBatch = 0;
   if(dogleg_gpu_device_count() <= 0) { dlb_set_error((fn + "no CUDA device available: libdogleg-b200 has no CPU fallback").c_str()); return -1; }
   if(!f || !p || !Nmeas || B == 0) { dlb_set_error((fn + "bad arguments (needs p, Nmeas, a callback and B > 0)").c_str()); return -1; }
@@ -1312,13 +1350,57 @@ extern "C" int dogleg_gpu_optimize_dense_batched_ragged(double* p, unsigned int 
     dlb_set_error((fn + "Nmeas[" + std::to_string(b) + "] = " + std::to_string(Nmeas[b]) + " exceeds INT_MAX").c_str());
     return -1;
   }
-  if(row_off[B] > (long long)(SIZE_MAX / sizeof(double) / (N + 1)))
+  // bytes per row: x and J
+  const size_t max_rows = form == BF_DENSE_RAGGED_F32 ? SIZE_MAX / (sizeof(double) + sizeof(float) * N)
+                                                      : SIZE_MAX / sizeof(double) / (N + 1);
+  if(row_off[B] > (long long)max_rows)
   {
     dlb_set_error((fn + "out of device memory").c_str());
     return -1;
   }
-  return batched_solve(BF_DENSE_RAGGED, p, N, 0, B, (void*)f, cookie, parameters, norm2x_out, iterations_out,
-                       returnBatch, Nmeas, row_off.data(), order.data());
+  return batched_solve(form, p, N, 0, B, f, cookie, parameters, norm2x_out, iterations_out, returnBatch, Nmeas,
+                       row_off.data(), order.data());
+}
+
+extern "C" int dogleg_gpu_optimize_dense_batched_ragged(double* p, unsigned int Nstate, const unsigned int* Nmeas,
+                                                        unsigned int B, dogleg_gpu_callback_dense_ragged_t* f,
+                                                        void* cookie, const dogleg_parameters2_t* parameters,
+                                                        double* norm2x_out, int* iterations_out,
+                                                        dogleg_gpu_batch_t** returnBatch)
+{
+  return ragged_solve(BF_DENSE_RAGGED, "dogleg_gpu_optimize_dense_batched_ragged", p, Nstate, Nmeas, B, (void*)f, cookie,
+                      parameters, norm2x_out, iterations_out, returnBatch);
+}
+
+extern "C" int dogleg_gpu_optimize_dense_batched_ragged_f32jac(double* p, unsigned int Nstate, const unsigned int* Nmeas,
+                                                               unsigned int B, dogleg_gpu_callback_dense_ragged_f32jac_t* f,
+                                                               void* cookie, const dogleg_parameters2_t* parameters,
+                                                               double* norm2x_out, int* iterations_out,
+                                                               dogleg_gpu_batch_t** returnBatch)
+{
+  return ragged_solve(BF_DENSE_RAGGED_F32, "dogleg_gpu_optimize_dense_batched_ragged_f32jac", p, Nstate, Nmeas, B,
+                      (void*)f, cookie, parameters, norm2x_out, iterations_out, returnBatch);
+}
+
+extern "C" int dogleg_gpu_optimize_dense_batched_f32jac(double* p, unsigned int Nstate, unsigned int Nmeas,
+                                                        unsigned int B, dogleg_gpu_callback_dense_batched_f32jac_t* f,
+                                                        void* cookie, const dogleg_parameters2_t* parameters,
+                                                        double* norm2x_out, int* iterations_out,
+                                                        dogleg_gpu_batch_t** returnBatch)
+{
+  static const std::string fn = "dogleg_gpu_optimize_dense_batched_f32jac: ";
+  if(returnBatch) *returnBatch = 0;
+  if(dogleg_gpu_device_count() <= 0) { dlb_set_error((fn + "no CUDA device available: libdogleg-b200 has no CPU fallback").c_str()); return -1; }
+  if(!f || !p || B == 0) { dlb_set_error((fn + "bad arguments (needs p, a callback and B > 0)").c_str()); return -1; }
+  const int N = (int)Nstate;
+  if(N > BT_NMAX || N < 1)
+  {
+    dlb_set_error((fn + "needs 1 <= Nstate <= 32; use dogleg_optimize_dense2 per problem for bigger ones").c_str());
+    return -1;
+  }
+  if(Nmeas > (unsigned int)INT_MAX) { dlb_set_error((fn + "Nmeas exceeds INT_MAX").c_str()); return -1; }
+  return batched_solve(BF_DENSE_F32, p, N, (int)Nmeas, B, (void*)f, cookie, parameters, norm2x_out, iterations_out,
+                       returnBatch);
 }
 
 extern "C" int dogleg_gpu_optimize_dense_products_batched2(double* p, unsigned int Nstate, unsigned int B,

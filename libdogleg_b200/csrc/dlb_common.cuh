@@ -130,3 +130,9 @@ __device__ __forceinline__ double ldg_stream(const double* p)
   asm volatile("ld.global.nc.L1::no_allocate.f64 %0, [%1];" : "=d"(v) : "l"(p));
   return v;
 }
+__device__ __forceinline__ float ldg_stream(const float* p)
+{
+  float v;
+  asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
+  return v;
+}

@@ -139,6 +139,12 @@ def load():
     L.dogleg_gpu_optimize_dense_batched_ragged.argtypes = [dp, C.c_uint, C.POINTER(C.c_uint), C.c_uint, vp, vp, PP, dp, ip,
                                                            C.POINTER(vp)]
     L.dogleg_gpu_optimize_dense_batched_ragged.restype = C.c_int
+    L.dogleg_gpu_optimize_dense_batched_f32jac.argtypes = [dp, C.c_uint, C.c_uint, C.c_uint, vp, vp, PP, dp, ip,
+                                                           C.POINTER(vp)]
+    L.dogleg_gpu_optimize_dense_batched_f32jac.restype = C.c_int
+    L.dogleg_gpu_optimize_dense_batched_ragged_f32jac.argtypes = [dp, C.c_uint, C.POINTER(C.c_uint), C.c_uint, vp, vp, PP,
+                                                                  dp, ip, C.POINTER(vp)]
+    L.dogleg_gpu_optimize_dense_batched_ragged_f32jac.restype = C.c_int
     L.dlb_batched_ragged_layout.argtypes = [C.POINTER(C.c_uint), C.c_uint, C.POINTER(C.c_longlong), ip]
     L.dlb_batched_ragged_layout.restype = C.c_int
     L.dogleg_gpu_batch_outlierness_ragged.argtypes = [vp, dp, dp, C.c_int, ip, ip, dp, dp]
