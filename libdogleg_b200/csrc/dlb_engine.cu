@@ -1937,11 +1937,12 @@ extern "C" int dlb_engine_debug_JtJ(dlb_engine_t* e, int s, double lambda, doubl
   if(e->type == DOGLEG_SPARSE)
   {
     if(assemble(e, L, true)) return -1;
-    // elements only, no elimination: lambda < 0 selects the test mode of the front kernel
+    // elements only, no elimination: lambda < 0 selects the test mode of the front kernel. This pass takes every
+    // front of a level, the fused leaf fronts of level 0 too, which level_rows does not count: size it for them
     const int nlev = (int)e->level_ptr.size() - 1;
     for(int l = 0; l < nlev; l++)
       dlb_launch_front_level(e->F, e->S, e->level_ptr[l], e->level_ptr[l+1], e->d_fronts, L.d_G, -1.0,
-                             e->d_minor, e->level_rows[l], 0, e->st);
+                             e->d_minor, l == 0 ? std::max(e->level_rows[0], e->leaf_max_rows) : e->level_rows[l], 0, e->st);
   }
   else if(dense_fill_front(e, L)) return -1;
   dlb_launch_fronts_to_dense(e->F, e->d_fronts, d_out, e->st);

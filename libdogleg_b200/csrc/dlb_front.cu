@@ -39,9 +39,10 @@ k_front_level(DlbFrontDev F, DlbSparseDev S, int l0, double* __restrict__ fronts
   const int tid = threadIdx.x;
 
   // Gpart == NULL: the front arrives pre-filled (dense solve types, row-sharded sums); else start
-  // from zero -- unless the children have already been gathered into it (large fronts, -2)
+  // from zero -- unless the children have already been gathered into it (large fronts, -2). A large
+  // front of 159 or 160 rows still fits the shared-memory variant: it then loads what was gathered.
   const long long toff = F.heavy_tmp_off ? F.heavy_tmp_off[s] : -1;
-  const bool gathered_in_place = toff == -2 && mode != 1 && !SMEM;
+  const bool gathered_in_place = toff == -2 && mode != 1;
   if(Gpart && !gathered_in_place) for(int idx = tid; idx < r * r; idx += NT) A[idx] = 0.0;
   else if(SMEM) for(int idx = tid; idx < r * r; idx += NT) A[idx] = Ag[idx];
   __syncthreads();
